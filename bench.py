@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: fp64 GPR loss+grad evaluations per second at N=32768, D=8 on B200 (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-points 32768]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-points 32768] [--dump-outputs DIR]
 
 One "step" = one full evaluation of model.loss() + loss.backward() for GPR with an Rbf-ARD kernel on the
 synthetic regression problem of BASELINE.md section 3 (covariance build, Cholesky, solves, log-det, and the
@@ -25,6 +25,11 @@ analytic gradient through (L L^T)^-1).  Prints ONE JSON line (rank 0).
                distributed exact GPR -- with their collectives; at --gpus 1 the single-GPU figures of the same runs.
 * --gpus N>1 : the headline GPR evaluation does not shard at this size (SURVEY 8e, DESIGN.md "replicas only"): every
                rank runs an independent replica; value = N * K / max-rank time.
+* --steps K  : the number of timed steps of every block of the line: value, e2e, int8_sliced_experimental and each
+               sharded configuration.
+* --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned to its caller -- the loss
+               and the gradient of every hyper-parameter -- as DIR/<name>.npy (float64), so that two builds can be
+               compared output for output (the inputs are seeded: the same arguments give the same inputs).
 """
 import argparse
 import json
@@ -66,7 +71,14 @@ def parse():
     ap.add_argument("--no-vendor-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
     ap.add_argument("--no-int8-sliced", action="store_true", help="skip the experimental int8-sliced engine block")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and gradients of the last timed step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def workload_config(n, world):
@@ -390,6 +402,13 @@ def one_eval(model):
     return loss
 
 
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def check_parity(n, loss_value, grads, fatal=True):
     """Loss (<= 1e-9) and gradients (<= 1e-7) of the timed evaluation against the unmodified reference's values at the
     named size; raises if the fast path has drifted -- a fast kernel whose results differ is not done.  (fatal=False:
@@ -458,6 +477,9 @@ def run_ours(args, rank, world, local_rank):
     grads = {"kernel.variance": model.kernel.variance.grad.cpu().numpy(),
              "kernel.length_scales": model.kernel.length_scales.grad.cpu().numpy(),
              "likelihood.variance": model.likelihood.variance.grad.cpu().numpy()}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss.detach().cpu().numpy(),
+                                         **{name + ".grad": g for name, g in grads.items()}})
     parity = check_parity(n, loss_value, grads)
 
     # ---------------- end-to-end through the public API with host inputs, all K steps ------------------------
@@ -498,7 +520,7 @@ def run_ours(args, rank, world, local_rank):
                 timer2 = nv.PhaseTimer()
                 nv.install_timer(timer2)
                 torch.cuda.synchronize()
-                k_steps = min(args.steps, 3)
+                k_steps = args.steps
                 f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 f0.record()
                 for _ in range(k_steps):
@@ -531,7 +553,7 @@ def run_ours(args, rank, world, local_rank):
     sharded = None
     if not args.no_sharded and n == 32768:
         import bench_sharded
-        sharded = bench_sharded.run(rank, world, device, ms_max / args.steps, parity.get("loss_pin"))
+        sharded = bench_sharded.run(rank, world, device, ms_max / args.steps, parity.get("loss_pin"), args.steps)
     if rank != 0:
         return
 

@@ -92,7 +92,7 @@ def _step(model, post=None):
     return loss.detach()
 
 
-def bench_vfe(rank, world, device, steps=3):
+def bench_vfe(rank, world, device, steps):
     per = VFE_SHARDS // world
     model = _vfe_model(range(rank * per, (rank + 1) * per), world > 1)
     _step(model)
@@ -105,7 +105,8 @@ def bench_vfe(rank, world, device, steps=3):
     phi = cond is not None and cond <= settings.vfe_phi_cond_max
     out = {"workload": "VFE Rbf-ARD fp64 N=%d D=%d M=%d loss+grad (configs[2]), rows sharded over %d rank(s)"
                        % (VFE_N, VFE_D, VFE_M, world),
-           "scaling": "strong", "ms_per_eval": ms, "evals_per_s": 1000.0 / ms, "rows_per_s": VFE_N / (ms / 1000.0),
+           "scaling": "strong", "steps": steps, "ms_per_eval": ms, "evals_per_s": 1000.0 / ms,
+           "rows_per_s": VFE_N / (ms / 1000.0),
            "loss": float(loss.item()),
            "form": ("Phi form, 3 N M^2 + 6 N M D flop executed (condition-gated: estimated cond_2(Kuu) = %.3g <= %.3g)"
                     % (cond, settings.vfe_phi_cond_max)) if phi else
@@ -147,7 +148,7 @@ def bench_vfe(rank, world, device, steps=3):
 # ------------------------------------------------------------------------------------------------------------
 # SVGP, configs[3]
 # ------------------------------------------------------------------------------------------------------------
-def bench_svgp(rank, world, device, steps=3):
+def bench_svgp(rank, world, device, steps):
     from gptorch_b200 import kernels, likelihoods
     from gptorch_b200.dist import allreduce_grads
     from gptorch_b200.models import SVGP
@@ -180,7 +181,7 @@ def bench_svgp(rank, world, device, steps=3):
         dist.all_reduce(hi, op=dist.ReduceOp.MAX)
     out = {"workload": "SVGP Matern52-ARD fp64 M=%d D=%d, minibatch %d per GPU x %d rank(s) (configs[3]; each rank's "
                        "shard of %d rows is resident in HBM)" % (SVGP_M, SVGP_D, SVGP_B, world, SVGP_ROWS),
-           "scaling": "weak", "ms_per_step": ms, "points_per_s": world * SVGP_B / (ms / 1000.0),
+           "scaling": "weak", "steps": steps, "ms_per_step": ms, "points_per_s": world * SVGP_B / (ms / 1000.0),
            "loss_rank0": float(loss.item()),
            "form": ("quadratic form (M x M algebra first), 3 B M^2 flop executed (condition-gated: estimated cond_2(Kuu) = "
                     "%.3g <= %.3g)" % (cond, settings.vfe_phi_cond_max)) if quad else
@@ -199,7 +200,7 @@ def bench_svgp(rank, world, device, steps=3):
 # ------------------------------------------------------------------------------------------------------------
 # distributed exact GPR, configs[1] strong-scaled and configs[4]
 # ------------------------------------------------------------------------------------------------------------
-def bench_dist_gpr(rank, world, device, n, single_gpu_ms=None, loss_pin=None, warm=True):
+def bench_dist_gpr(rank, world, device, n, steps, single_gpu_ms=None, loss_pin=None, warm=True):
     from bench import synth_regression
     from gptorch_b200 import kernels, likelihoods
     from gptorch_b200.models import DistributedGPR
@@ -213,25 +214,25 @@ def bench_dist_gpr(rank, world, device, n, single_gpu_ms=None, loss_pin=None, wa
     dg.WAIT_LOG = []
     timer = nv.PhaseTimer()
     nv.install_timer(timer)
-    ms, loss = _timed(lambda: _step(model), 1, world, device)
+    ms, loss = _timed(lambda: _step(model), steps, world, device)
     nv.install_timer(None)
     stages = timer.totals_ms()
     waits, dg.WAIT_LOG = dg.WAIT_LOG, None
     wait_ms = [a.elapsed_time(b) for a, b in waits]
-    wait = torch.tensor([sum(wait_ms)], dtype=torch.float64, device=device)
+    wait = torch.tensor([sum(wait_ms) / steps], dtype=torch.float64, device=device)       # per evaluation
     if world > 1:
         dist.all_reduce(wait, op=dist.ReduceOp.MAX)
     panels = (n + 1023) // 1024
     out = {"workload": "exact GPR Rbf-ARD fp64 N=%d D=8 loss+grad, block-column-cyclic Cholesky + inverse + gradient over "
                        "%d rank(s), 1024-column panels" % (n, world),
-           "scaling": "strong", "ms_per_eval": ms, "loss": float(loss.item()),
+           "scaling": "strong", "steps": steps, "ms_per_eval": ms, "loss": float(loss.item()),
            "tflops_aggregate": float(n) ** 3 / (ms / 1000.0) / 1e12,
            "frac_of_aggregate_fp64_peak": float(n) ** 3 / (ms / 1000.0) / 1e12 / (world * FP64_PEAK_TFLOPS),
            "collectives": "ncclBroadcast of each factored panel ((N - c) x 1024 doubles) in 3 sweeps (L, T = L^-1, Kinv), "
                           "all_reduce of a (N doubles) and of D + 2 gradient doubles",
-           "stage_ms_rank0": {k: v for k, v in sorted(stages.items()) if k.startswith("dist_")},
-           "stage_note": "dist_potrf / dist_trtri / dist_lauum are N^3/3 flop each, spread over the ranks",
-           "panel_wait_ms_total_max_rank": wait.item(), "panel_waits": len(wait_ms),
+           "stage_ms_rank0": {k: v / steps for k, v in sorted(stages.items()) if k.startswith("dist_")},
+           "stage_note": "dist_potrf / dist_trtri / dist_lauum are N^3/3 flop each, spread over the ranks; per evaluation",
+           "panel_wait_ms_total_max_rank": wait.item(), "panel_waits": len(wait_ms) // steps,
            "panel_wait_ms_per_panel": wait.item() / max(3 * panels, 1),
            "max_mem_gb": torch.cuda.max_memory_allocated() / 1e9}
     if single_gpu_ms:
@@ -245,15 +246,15 @@ def bench_dist_gpr(rank, world, device, n, single_gpu_ms=None, loss_pin=None, wa
     return out
 
 
-def run(rank, world, device, single_gpu_ms, loss_pin, budget_s=240.0):
-    """The `sharded` block of bench.py's JSON line."""
+def run(rank, world, device, single_gpu_ms, loss_pin, steps, budget_s=240.0):
+    """The `sharded` block of bench.py's JSON line; every configuration times `steps` steps (bench.py --steps)."""
     t0 = time.perf_counter()
     out = {"n_gpus": world}
-    out["vfe"] = bench_vfe(rank, world, device)
-    out["svgp"] = bench_svgp(rank, world, device)
+    out["vfe"] = bench_vfe(rank, world, device, steps)
+    out["svgp"] = bench_svgp(rank, world, device, steps)
     if world > 1:
-        out["dist_gpr_n32768"] = bench_dist_gpr(rank, world, device, 32768, single_gpu_ms, loss_pin)
+        out["dist_gpr_n32768"] = bench_dist_gpr(rank, world, device, 32768, steps, single_gpu_ms, loss_pin)
     if world >= 8 and time.perf_counter() - t0 < budget_s:
-        out["dist_gpr_n131072"] = bench_dist_gpr(rank, world, device, C5_N, None, C5_LOSS_R01, warm=False)
+        out["dist_gpr_n131072"] = bench_dist_gpr(rank, world, device, C5_N, steps, None, C5_LOSS_R01, warm=False)
     out["seconds"] = time.perf_counter() - t0
     return out

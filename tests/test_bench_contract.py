@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -29,6 +32,42 @@ def test_reference_arm_prints_the_contract_line():
     assert d["metric"] == bench.METRIC and d["config"] == bench.workload_config(32768, 1)
     assert "N=32768" in d["config"]["workload"] and "inputs_exceed_l2" in d["config"]["l2"]
     assert d["ms_per_step"] < d["ms_per_step_full_size_extrapolated"]
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(args, tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True,
+                         timeout=300, cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr, out.stderr[-2000:]
+    assert not out.stdout.strip() and not os.listdir(tmp_path)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: the loss and the three hyper-parameter gradients of the last timed step, float64, equal to the
+    oracle's on the same seeded inputs (and to the reference's loss pin at this size); --steps is the timed step count."""
+    sys.path.insert(0, ROOT)
+    from oracle import gp_oracle as O
+    n, dump = 2048, tmp_path / "dump"
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--num-points", str(n), "--steps", "2",
+                          "--warmup", "1", "--no-cpu-baseline", "--no-vendor-baseline", "--no-sharded",
+                          "--no-int8-sliced", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=900, cwd=tmp_path)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+    assert line["steps"] == 2 and line["e2e"]["steps"] == 2
+    got = {f[:-len(".npy")]: np.load(dump / f) for f in os.listdir(dump)}
+    assert set(got) == {"loss", "kernel.variance.grad", "kernel.length_scales.grad", "likelihood.variance.grad"}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["loss"].shape == (1,) and got["loss"][0] == line["loss"]
+    assert abs(got["loss"][0] - -1420.2752146205817) <= 1e-9 * 1420.3          # BASELINE.md section 3 pin
+    X, Y, _ = O.synth_regression(n, 8)
+    ref_loss, ref = O.gpr_loss_and_grads("Rbf", X, Y, np.ones(8), 1.0, 0.01)
+    rel = lambda a, b: float(np.abs(a - b).max() / np.abs(b).max())  # noqa: E731
+    assert rel(got["loss"], ref_loss.numpy()) <= 1e-9
+    assert rel(got["kernel.variance.grad"], ref["variance"].numpy()) <= 1e-7
+    assert rel(got["kernel.length_scales.grad"], ref["length_scales"].numpy()) <= 1e-7
+    assert rel(got["likelihood.variance.grad"], ref["noise"].numpy()) <= 1e-7
 
 
 def test_sharded_bench_module_is_importable_without_a_gpu():
