@@ -507,6 +507,7 @@ class GPRLogLikFn(Function):
               gptorch/functions.py:28-43) -> alpha = L^-1 resid -> -1/2 |alpha|^2 - dy sum log L_ii - const.
     backward: a = L^-T alpha ; Kinv = potri(L) in place ; W = 1/2 (dy Kinv - a a^T) reduced against
               dK/d(ell, sigma2) on the fly ; d/d noise = tr W ; d/d resid = -a.       (SURVEY 10)
+              When X requires a gradient, a second pass reduces the same W against dK/dX (gpb_gpr_grad's gX).
     One N^2 buffer in total; N^3/3 + 2N^3/3 flops.
     """
 
@@ -549,15 +550,17 @@ class GPRLogLikFn(Function):
             nv.trsv_(buf, dinv, a, True)                 # a = Ky^-1 resid
         with nv.phase("potri"):
             kd = nv.potri_(buf, ctx.ld, dinv)            # Kinv, in place (L is gone after this)
+        gX = torch.empty_like(X) if ctx.needs_input_grad[1] else None
         with nv.phase("gpr_grad"):
-            g_ell, g_s2, g_noise = nv.gpr_grad(ctx.kind, X, ell, sigma2, buf, ctx.ld, kd, a)
+            g_ell, g_s2, g_noise = nv.gpr_grad(ctx.kind, X, ell, sigma2, buf, ctx.ld, kd, a, gX=gX)
         g = g.reshape(())
         # the native reduction returns d(-loglik)/d theta; the node's output is +loglik
         out_ell = (-g) * g_ell.reshape(ell.shape) if ctx.needs_input_grad[3] else None
         out_s2 = (-g) * g_s2.reshape(sigma2.shape) if (sigma2 is not None and ctx.needs_input_grad[4]) else None
         out_noise = (-g) * g_noise.reshape(-1) if ctx.needs_input_grad[5] else None
         out_resid = (-g) * a if ctx.needs_input_grad[2] else None
-        return None, None, out_resid, out_ell, out_s2, out_noise
+        out_x = (-g) * gX if gX is not None else None
+        return None, out_x, out_resid, out_ell, out_s2, out_noise
 
 
 class GPRCompositeLogLikFn(Function):
@@ -607,11 +610,12 @@ class GPRCompositeLogLikFn(Function):
             W = nv.potri_assemble(buf, ctx.ld, kd)                                   # full symmetric Ky^-1
         with nv.phase("gpr_grad"):
             nv.gemm(nv.GEMM_NT, a, a, alpha=-0.5, beta=0.5 * dy, C=W)                # W = 1/2 (dy Kinv - a a^T)
-            grads, _, _ = _composite_grads(ctx.spec, X, None, params, W, False, False)
+            grads, gX, _ = _composite_grads(ctx.spec, X, None, params, W, ctx.needs_input_grad[1], False)
             g_noise = W.diagonal().sum().reshape(1)
         g = g.reshape(())
         need = ctx.needs_input_grad
-        return (None, None, (-g) * a if need[2] else None, (-g) * g_noise if need[3] else None) + tuple(
+        out_x = (-g) * gX if gX is not None else None
+        return (None, out_x, (-g) * a if need[2] else None, (-g) * g_noise if need[3] else None) + tuple(
             ((-g) * gr if (gr is not None and need[4 + i]) else None) for i, gr in enumerate(grads))
 
 
@@ -742,9 +746,12 @@ class VfeStatsFn(Function):
             R = nv.gemm(nv.GEMM_NN, T, R, flags=nv.GF_KLO_M)   # L^-T S L^-1  (T[m][k] = 0 for k < m)
         w = nv.gemm(nv.GEMM_NN, T, gAY)          # L^-T gAY   (m x dy)
         panels, ctx.panels = ctx.panels, None
+        # dLoss/dX: each chunk's panel gradient reduced with X and Z exchanged.  The rows are this rank's own, so it is
+        # not all-reduced; sum Kdiag = n sigma2 does not depend on X.
+        gX = torch.empty_like(X) if ctx.needs_input_grad[1] else None
         if phi:
             with nv.phase("vfe_stats_bwd"):      # ONE native call re-streams the chunks (gpb_kuf_stats_bwd)
-                g_ell, g_s2, gZ = nv.kuf_stats_bwd(kind, X, Y, Z, ell, sigma2, chunk, R, w, kfu=panels)
+                g_ell, g_s2, gZ = nv.kuf_stats_bwd(kind, X, Y, Z, ell, sigma2, chunk, R, w, kfu=panels, gX=gX)
             del panels
         else:
             g_ell = torch.zeros_like(ell.reshape(-1))
@@ -763,6 +770,8 @@ class VfeStatsFn(Function):
                 del P
                 with nv.phase("vfe_kern_bwd"):
                     ge, gs, gz = nv.kern_bwd(kind, X[s:e], Z, ell, sigma2, G, True)
+                    if gX is not None:
+                        gX[s:e] = nv.kern_bwd(kind, Z, X[s:e], ell, sigma2, G, True, g_transposed=True)[2]
                 del G
                 g_ell += ge
                 g_s2 += gs
@@ -776,7 +785,7 @@ class VfeStatsFn(Function):
         nv.gemm(nv.GEMM_NT, gAY, AY, beta=1.0, C=Q)
         gL = nv.gemm(nv.GEMM_NN, T, Q, alpha=-1.0, flags=nv.GF_KLO_M)
         gL.tril_()
-        return (None, None, None, gZ if ctx.needs_input_grad[3] else None,
+        return (None, gX, None, gZ if ctx.needs_input_grad[3] else None,
                 g_ell.reshape(ell.shape) if ctx.needs_input_grad[4] else None,
                 g_s2.reshape(sigma2.shape) if (sigma2 is not None and ctx.needs_input_grad[5]) else None,
                 gL if ctx.needs_input_grad[6] else None, None, None, None)

@@ -68,17 +68,17 @@ SIGNATURES = {
     "gpb_ozaki_config": (c_int, [c_int]),
     "gpb_gemm_splitk": (c_int, [c_int, c_int, c_int, c_int, c_int, c_double, c_void_p, c_long, c_void_p, c_long, c_double,
                                 c_void_p, c_long, c_long, c_int, c_void_p]),
-    "gpb_kuf_stats_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "gpb_kuf_stats_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
     "gpb_kuf_stats_fwd": (c_int, [c_int, c_void_p, c_long, c_long, c_void_p, c_int, c_long, c_void_p, c_int, c_long, c_int,
                                   c_void_p, c_int, c_void_p, c_int, c_void_p, c_long, c_void_p, c_long, c_void_p, c_long,
                                   c_void_p, c_size_t, c_void_p]),
     "gpb_kuf_stats_bwd": (c_int, [c_int, c_void_p, c_long, c_long, c_void_p, c_int, c_long, c_void_p, c_int, c_long, c_int,
                                   c_void_p, c_int, c_void_p, c_int, c_void_p, c_long, c_void_p, c_long, c_void_p, c_long,
-                                  c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+                                  c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_long]),
     "gpb_gpr_grad_workspace_bytes": (c_size_t, [c_int, c_int]),
     "gpb_gpr_grad": (c_int, [c_int, c_void_p, c_int, c_long, c_int, c_void_p, c_int, c_void_p, c_void_p, c_long,
                              c_void_p, c_void_p, c_int, c_long, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
-                             c_void_p]),
+                             c_void_p, c_void_p, c_long]),
 }
 
 _ERRORS = {-1: "bad argument", -2: "alignment (16-byte base, even leading dimension required)",

@@ -502,7 +502,7 @@ def kuf_stats_fwd(kind, X, Y, Z, ell, sigma2, chunk, cache=False):
     ell = _c(ell).reshape(-1)
     s2 = _c(sigma2).reshape(-1)
     chunk = int(max(1, min(chunk, max(n, 1))))
-    ws = _ws(query("gpb_kuf_stats_workspace_bytes", m, D, dy, chunk), X.device)
+    ws = _ws(query("gpb_kuf_stats_workspace_bytes", m, D, dy, chunk, 0), X.device)
     Phi = _aligned_empty(m, m, X.device)[0]
     psi = torch.empty((m, dy), dtype=torch.float64, device=X.device)
     kfu = _aligned_empty(n, m, X.device)[0] if cache else None
@@ -512,8 +512,9 @@ def kuf_stats_fwd(kind, X, Y, Z, ell, sigma2, chunk, cache=False):
     return Phi[:, :m], psi, kfu
 
 
-def kuf_stats_bwd(kind, X, Y, Z, ell, sigma2, chunk, R, W, kfu=None):
-    """(g_ell, g_sigma2, gZ): the gradient Kfu_c R + Y_c W^T of every panel reduced against dK/d(ell, sigma2, Z)."""
+def kuf_stats_bwd(kind, X, Y, Z, ell, sigma2, chunk, R, W, kfu=None, gX=None):
+    """(g_ell, g_sigma2, gZ): the gradient Kfu_c R + Y_c W^T of every panel reduced against dK/d(ell, sigma2, Z).
+    gX (n x D, optional) receives the gradient with respect to X."""
     X, Y, Z = _c(X), _c(Y), _c(Z)
     n, D = X.shape
     m, dy = Z.shape[0], Y.shape[1]
@@ -521,19 +522,21 @@ def kuf_stats_bwd(kind, X, Y, Z, ell, sigma2, chunk, R, W, kfu=None):
     s2 = _c(sigma2).reshape(-1)
     R, W = _gemm_operand(R), _c(W)
     chunk = int(max(1, min(chunk, max(n, 1))))
-    ws = _ws(query("gpb_kuf_stats_workspace_bytes", m, D, dy, chunk), X.device)
+    ws = _ws(query("gpb_kuf_stats_workspace_bytes", m, D, dy, chunk, 1 if gX is not None else 0), X.device)
     g_ell = torch.empty(ell.numel(), dtype=torch.float64, device=X.device)
     g_s2 = torch.empty(1, dtype=torch.float64, device=X.device)
     gZ = torch.empty((m, D), dtype=torch.float64, device=X.device)
     call("gpb_kuf_stats_bwd", kind, ptr(X), n, X.stride(0), ptr(Y), dy, Y.stride(0), ptr(Z), m, Z.stride(0), D, ptr(ell),
          ell.numel(), ptr(s2), chunk, ptr(R), R.stride(0), ptr(W), W.stride(0), ptr(kfu),
-         kfu.stride(0) if kfu is not None else 0, ptr(g_ell), ptr(g_s2), ptr(gZ), ptr(ws), ws.numel() * 8, stream_ptr())
+         kfu.stride(0) if kfu is not None else 0, ptr(g_ell), ptr(g_s2), ptr(gZ), ptr(ws), ws.numel() * 8, stream_ptr(),
+         ptr(gX), gX.stride(0) if gX is not None else 0)
     return g_ell, g_s2, gZ
 
 
 # ---------------------------------------------------------------------------------------------- fused GPR gradient
-def gpr_grad(kind, X, ell, sigma2, Kinv, ldk, kd, a):
-    """Returns (g_ell, g_sigma2, g_noise): d loss / d (ell, sigma2, sigma_n^2) for the GPR loss."""
+def gpr_grad(kind, X, ell, sigma2, Kinv, ldk, kd, a, gX=None):
+    """Returns (g_ell, g_sigma2, g_noise): d loss / d (ell, sigma2, sigma_n^2) for the GPR loss.  gX (n x D, optional)
+    receives d loss / dX."""
     X = _c(X)
     n, D = X.shape
     ell = _c(ell).reshape(-1)
@@ -545,5 +548,6 @@ def gpr_grad(kind, X, ell, sigma2, Kinv, ldk, kd, a):
     ws = _ws(ws_bytes, X.device)
     call("gpb_gpr_grad", kind, ptr(X), n, X.stride(0), D, ptr(ell), ell.numel(),
          ptr(_c(sigma2).reshape(-1)) if sigma2 is not None else None, ptr(Kinv), ldk, ptr(kd), ptr(a), a.shape[1],
-         a.stride(0), ptr(g_ell), ptr(g_sig), ptr(g_noise), ptr(ws), ws.numel() * 8, stream_ptr())
+         a.stride(0), ptr(g_ell), ptr(g_sig), ptr(g_noise), ptr(ws), ws.numel() * 8, stream_ptr(),
+         ptr(gX), gX.stride(0) if gX is not None else 0)
     return g_ell, g_sig, g_noise

@@ -59,7 +59,7 @@ size_t gpr_grad_workspace_bytes(int n, int D);
 int gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* ell, int ell_len,
              const double* sigma2, const double* Kinv, long ldk, const double* kdiag_blocks, const double* a,
              int dy, long lda_a, double* g_ell, double* g_sigma2, double* g_noise, void* workspace,
-             size_t workspace_bytes, cudaStream_t stream);
+             size_t workspace_bytes, double* gX, long ldgx, cudaStream_t stream);
 }  // namespace gpb
 
 using namespace gpb;
@@ -136,7 +136,7 @@ static inline int kuf_k_per_split(int rows) {
 #pragma GCC visibility push(default)
 extern "C" {
 
-int gpb_version(void) { return 100; }
+int gpb_version(void) { return 101; }
 const char* gpb_last_error(void) { return last_error(); }
 int gpb_block_size(void) { return NB; }
 long gpb_launch_count(void) { return launch_count(); }
@@ -308,8 +308,22 @@ int gpb_gemm_splitk(int mode, int m, int n, int k_total, int k_per_split, double
   return gemm_launch(gm, mapA, mapB, g, S(stream));
 }
 
+// kern_bwd scratch of the input-gradient reduction K(Z, X_c): the largest over every chunk height up to chunk_rows (a
+// short last chunk has fewer column blocks and may take more strips).  For a fixed number of 128-column blocks the size
+// grows with the height, so the block-aligned heights and chunk_rows itself cover all cases.
+static size_t kuf_gx_kb_bytes(int m, int chunk_rows, int D) {
+  size_t b = 0;
+  for (int r = 128;; r += 128) {
+    const int h = std::min(r, chunk_rows);
+    b = std::max(b, kern_bwd_workspace_bytes(m, h, D));
+    if (h == chunk_rows) break;
+  }
+  return b;
+}
+
 // Workspace: [3 chunk x ldm buffers][split slots S x m x ldm][kern_bwd scratch][gemv_t scratch][small temporaries]
-size_t gpb_kuf_stats_workspace_bytes(int m, int D, int dy, int chunk_rows) {
+// and, with the input gradient, [kern_bwd scratch of the transposed reduction][chunk x D gradient, D + 1 temporaries]
+size_t gpb_kuf_stats_workspace_bytes(int m, int D, int dy, int chunk_rows, int with_gx) {
   if (m <= 0 || D <= 0 || dy <= 0 || chunk_rows <= 0) return 0;
   const size_t ldm = static_cast<size_t>(m) + (m & 1);
   size_t b = 3 * kuf_align(static_cast<size_t>(chunk_rows) * ldm * 8);       // two pipeline buffers + one panel
@@ -317,6 +331,10 @@ size_t gpb_kuf_stats_workspace_bytes(int m, int D, int dy, int chunk_rows) {
   b += kuf_align(kern_bwd_workspace_bytes(chunk_rows, m, D));
   b += kuf_align(gemv_t_workspace_bytes(chunk_rows, m));
   b += kuf_align((static_cast<size_t>(D) + 1 + static_cast<size_t>(m) * D) * 8);
+  if (with_gx) {
+    b += kuf_align(kuf_gx_kb_bytes(m, chunk_rows, D));
+    b += kuf_align((static_cast<size_t>(chunk_rows) * D + D + 1) * 8);
+  }
   return b;
 }
 
@@ -327,7 +345,7 @@ int gpb_kuf_stats_fwd(int kind, const double* X, long n, long ldx, const double*
   if (n < 0 || m <= 0 || D <= 0 || dy <= 0 || chunk_rows <= 0) return GPB_ERR_BADARG;
   if (!X || !Y || !Z || !ell || !sigma2 || !Phi || !psi || ldphi < m || ldpsi < dy) return GPB_ERR_BADARG;
   if (kfu_cache && (ldcache < m || (ldcache & 1) || (reinterpret_cast<uintptr_t>(kfu_cache) & 15))) return GPB_ERR_ALIGN;
-  if (!workspace || workspace_bytes < gpb_kuf_stats_workspace_bytes(m, D, dy, chunk_rows)) return GPB_ERR_BADARG;
+  if (!workspace || workspace_bytes < gpb_kuf_stats_workspace_bytes(m, D, dy, chunk_rows, 0)) return GPB_ERR_BADARG;
   if (reinterpret_cast<uintptr_t>(workspace) & 15) return GPB_ERR_ALIGN;
   const long ldm = m + (m & 1);
   const size_t chunk_bytes = kuf_align(static_cast<size_t>(chunk_rows) * ldm * 8);
@@ -379,12 +397,14 @@ int gpb_kuf_stats_bwd(int kind, const double* X, long n, long ldx, const double*
                       int m, long ldz, int D, const double* ell, int ell_len, const double* sigma2, int chunk_rows,
                       const double* R, long ldr, const double* W, long ldw, const double* kfu_cache, long ldcache,
                       double* g_ell, double* g_sigma2, double* gZ, void* workspace, size_t workspace_bytes,
-                      void* stream) {
+                      void* stream, double* gX, long ldgx) {
   if (n < 0 || m <= 0 || D <= 0 || dy <= 0 || chunk_rows <= 0) return GPB_ERR_BADARG;
   if (!X || !Y || !Z || !ell || !sigma2 || !R || !W || !g_ell || !g_sigma2 || !gZ) return GPB_ERR_BADARG;
+  if (gX && ldgx < D) return GPB_ERR_BADARG;
   if (ldr < m || (ldr & 1) || (reinterpret_cast<uintptr_t>(R) & 15)) return GPB_ERR_ALIGN;
   if (kfu_cache && (ldcache < m || (ldcache & 1) || (reinterpret_cast<uintptr_t>(kfu_cache) & 15))) return GPB_ERR_ALIGN;
-  if (!workspace || workspace_bytes < gpb_kuf_stats_workspace_bytes(m, D, dy, chunk_rows)) return GPB_ERR_BADARG;
+  if (!workspace || workspace_bytes < gpb_kuf_stats_workspace_bytes(m, D, dy, chunk_rows, gX != nullptr))
+    return GPB_ERR_BADARG;
   if (reinterpret_cast<uintptr_t>(workspace) & 15) return GPB_ERR_ALIGN;
   const long ldm = m + (m & 1);
   const size_t chunk_bytes = kuf_align(static_cast<size_t>(chunk_rows) * ldm * 8);
@@ -400,6 +420,14 @@ int gpb_kuf_stats_bwd(int kind, const double* X, long n, long ldx, const double*
   double* t_ell = reinterpret_cast<double*>(w);
   double* t_s2 = t_ell + D;
   double* t_z = t_s2 + 1;
+  w += kuf_align((static_cast<size_t>(D) + 1 + static_cast<size_t>(m) * D) * 8);
+  // input gradient: the same G_c reduced with the roles of X and Z exchanged (G_c read transposed), whose column
+  // gradient is dLoss/dX_c; its hyper-parameter sums are discarded
+  void* xb_ws = w;
+  const size_t xb_bytes = gX ? kuf_gx_kb_bytes(m, chunk_rows, D) : 0;
+  double* x_g = reinterpret_cast<double*>(w + kuf_align(xb_bytes));
+  double* x_ell = x_g + static_cast<size_t>(chunk_rows) * D;
+  double* x_s2 = x_ell + D;
   cudaStream_t st = S(stream);
   KufAux* aux = nullptr;
   if (int rc = kuf_aux(st, &aux)) return rc;
@@ -440,6 +468,13 @@ int gpb_kuf_stats_bwd(int kind, const double* X, long n, long ldx, const double*
     kuf_accumulate_kernel<<<(m * D + 255) / 256, 256, 0, aux->side>>>(gZ, t_z, static_cast<long>(m) * D);
     count_launch(3);
     GPB_CUDA_CHECK(cudaGetLastError());
+    if (gX) {
+      rc = gpb_kern_bwd(kind, Z, m, ldz, X + s0 * ldx, rows, ldx, D, ell, ell_len, sigma2, G, ldm, 1, x_ell, x_s2, x_g,
+                        xb_ws, xb_bytes, aux->side);
+      if (rc) return rc;
+      GPB_CUDA_CHECK(cudaMemcpy2DAsync(gX + s0 * ldgx, ldgx * 8, x_g, static_cast<size_t>(D) * 8,
+                                       static_cast<size_t>(D) * 8, rows, cudaMemcpyDeviceToDevice, aux->side));
+    }
     GPB_CUDA_CHECK(cudaEventRecord(aux->free_[b], aux->side));
   }
   GPB_CUDA_CHECK(cudaEventRecord(aux->join, aux->side));
@@ -451,9 +486,9 @@ size_t gpb_gpr_grad_workspace_bytes(int n, int D) { return gpr_grad_workspace_by
 int gpb_gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* ell, int ell_len,
                  const double* sigma2, const double* Kinv, long ldk, const double* kdiag_blocks, const double* a,
                  int dy, long lda_a, double* g_ell, double* g_sigma2, double* g_noise, void* workspace,
-                 size_t workspace_bytes, void* stream) {
+                 size_t workspace_bytes, void* stream, double* gX, long ldgx) {
   return gpr_grad(kind, X, n, ldx, D, ell, ell_len, sigma2, Kinv, ldk, kdiag_blocks, a, dy, lda_a, g_ell, g_sigma2,
-                  g_noise, workspace, workspace_bytes, S(stream));
+                  g_noise, workspace, workspace_bytes, gX, ldgx, S(stream));
 }
 
 }  // extern "C"

@@ -834,14 +834,184 @@ size_t gpr_grad_workspace_bytes(int n, int D) {
   return static_cast<size_t>(ncb) * strips * (D + 2) * sizeof(double) + 256;
 }
 
+// ================================================================================================
+// input gradient of the fused GPR loss
+// ================================================================================================
+// gX_t = sum_s 2 W_ts dK_ts/dx_t with W = 1/2 (dy Kinv - a a^T) formed on the fly from the blocked lower Kinv
+// (W_ts = W_st: the pair is read from row max(t, s), column min(t, s)).  One CTA owns 128 target rows (one per thread
+// pair, the two halves take alternate source rows) and one chunk of KB_DC feature dimensions (blockIdx.y), and sweeps
+// EVERY source row: each pair of the lower triangle is visited twice, once per end, so each target's sum is complete
+// inside its CTA and is combined in a fixed order -- no per-CTA partials, no workspace, deterministic.
+//   stationary: dK_ts/dx_td = -sigma2 fac1(r2) (x~_td - x~_sd) / ell_d   (the g_ell reduction's fac1; zero below the
+//               r2 clamp, gptorch/kernels.py:171-172, so coincident points contribute nothing)
+//   Linear:     dK_ts/dx_td = v_d x_sd  (the diagonal pair included: dK_tt/dx_t = 2 v x_t)
+template <int KB_DC, int KIND>
+__global__ void __launch_bounds__(KB_THREADS, 2) gpr_gx_kernel(const KbwdParams p, double* __restrict__ gX, long ldgx) {
+  const int kind = KIND >= 0 ? KIND : p.kind;
+  extern __shared__ double kb_smem[];
+  const int D = p.D;
+  double* Xts = kb_smem;                                   // [D][128] target coordinates (scaled)
+  double* Xss = Xts + static_cast<size_t>(D) * KB_COLS;    // [KB_ROWS][D] source coordinates (scaled)
+  double* ellv = Xss + static_cast<size_t>(KB_ROWS) * D;   // [D]
+  double* at = ellv + D;                                   // [KB_DY][128]
+  double* as = at + KB_COLS * KB_DY;                       // [KB_ROWS][KB_DY]
+  double* comb = as + KB_ROWS * KB_DY + 32;                // [2][128]
+
+  const int t = threadIdx.x, c = t & 127, half = t >> 7;
+  const int c0 = blockIdx.x * KB_COLS;
+  const int j = c0 + c;                                    // target row
+  const bool jvalid = j < p.n1;
+  const int d0 = blockIdx.y * KB_DC;
+  const bool linear = kind == KERN_LINEAR;
+
+  for (int d = t; d < D; d += KB_THREADS) ellv[d] = p.ell[p.ell_len == 1 ? 0 : d];
+  __syncthreads();
+  for (int idx = t; idx < KB_COLS * D; idx += KB_THREADS) {
+    const int cc = idx / D, d = idx - cc * D;
+    double v = 0.0;
+    if (c0 + cc < p.n1) {
+      v = p.X1[static_cast<long>(c0 + cc) * p.ldx1 + d];
+      if (!linear) v /= ellv[d];
+    }
+    Xts[d * KB_COLS + cc] = v;
+  }
+  const double sig2 = linear ? 1.0 : *p.sigma2;
+
+  double acc[KB_DC];
+#pragma unroll
+  for (int dd = 0; dd < KB_DC; ++dd) acc[dd] = 0.0;
+
+  for (int rc = 0; rc < p.nrc; ++rc) {
+    const int i0 = rc * KB_ROWS;
+    __syncthreads();
+    for (int idx = t; idx < KB_ROWS * D; idx += KB_THREADS) {
+      const int rr = idx / D, d = idx - rr * D;
+      double v = 0.0;
+      if (i0 + rr < p.n1) {
+        v = p.X1[static_cast<long>(i0 + rr) * p.ldx1 + d];
+        if (!linear) v /= ellv[d];
+      }
+      Xss[rr * D + d] = v;
+    }
+    // aa[rr] = sum_o a[s][o] a[t][o], staged in chunks of KB_DY outputs
+    double hreg[KB_RT];
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) hreg[rr] = 0.0;
+    for (int o0 = 0; o0 < p.dy; o0 += KB_DY) {
+      __syncthreads();
+      for (int idx = t; idx < KB_COLS * KB_DY; idx += KB_THREADS) {
+        const int cc = idx / KB_DY, o = idx - cc * KB_DY;
+        at[o * KB_COLS + cc] = (c0 + cc < p.n1 && o0 + o < p.dy) ? p.a[static_cast<long>(c0 + cc) * p.lda + o0 + o] : 0.0;
+      }
+      for (int idx = t; idx < KB_ROWS * KB_DY; idx += KB_THREADS) {
+        const int rr = idx / KB_DY, o = idx - rr * KB_DY;
+        as[idx] = (i0 + rr < p.n1 && o0 + o < p.dy) ? p.a[static_cast<long>(i0 + rr) * p.lda + o0 + o] : 0.0;
+      }
+      __syncthreads();
+#pragma unroll
+      for (int o = 0; o < KB_DY; ++o) {
+        const double aj = at[o * KB_COLS + c];
+#pragma unroll
+        for (int rr = 0; rr < KB_RT; ++rr) hreg[rr] += as[(half * KB_RT + rr) * KB_DY + o] * aj;
+      }
+    }
+    __syncthreads();
+
+    double r2[KB_RT];
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) r2[rr] = 0.0;
+    if (!linear) {
+      for (int d = 0; d < D; ++d) {
+        const double xt = Xts[d * KB_COLS + c];
+#pragma unroll
+        for (int rr = 0; rr < KB_RT; ++rr) {
+          const double diff = Xss[(half * KB_RT + rr) * D + d] - xt;
+          r2[rr] += diff * diff;
+        }
+      }
+    }
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) {
+      const int i = i0 + half * KB_RT + rr;
+      double h = 0.0;
+      if (jvalid && i < p.n1) {
+        const int hi = i > j ? i : j, lo = i > j ? j : i;
+        const bool same_blk = (hi / NB) == (lo / NB);
+        const double kinv = same_blk ? p.kd[static_cast<long>(hi) * NB + (lo - (lo / NB) * NB)]
+                                     : p.Kinv[static_cast<long>(hi) * p.ldk + lo];
+        const double g = 2.0 * (0.5 * (static_cast<double>(p.dy) * kinv - hreg[rr]));
+        if (linear) {
+          h = g;
+        } else {
+          double kbase, fac1;
+          kern_base_fac(kind, r2[rr], kbase, fac1);
+          h = g * fac1 * sig2;
+        }
+      }
+      hreg[rr] = h;
+    }
+#pragma unroll
+    for (int dd = 0; dd < KB_DC; ++dd) {
+      const int d = d0 + dd;
+      if (d < D) {
+        const double xt = Xts[d * KB_COLS + c];
+#pragma unroll
+        for (int rr = 0; rr < KB_RT; ++rr) {
+          const double xs = Xss[(half * KB_RT + rr) * D + d];
+          acc[dd] += linear ? hreg[rr] * xs : hreg[rr] * (xs - xt);
+        }
+      }
+    }
+  }
+
+  // the two halves' sums of each target, in a fixed order; then the 1/ell (stationary) or v (Linear) factor
+#pragma unroll
+  for (int dd = 0; dd < KB_DC; ++dd) {
+    const int d = d0 + dd;
+    if (d >= D) break;  // uniform across the block
+    __syncthreads();
+    comb[half * KB_COLS + c] = acc[dd];
+    __syncthreads();
+    if (half == 0 && jvalid) {
+      const double s = comb[c] + comb[KB_COLS + c];
+      gX[static_cast<long>(j) * ldgx + d] = linear ? s * ellv[d] : s / ellv[d];
+    }
+  }
+}
+
+template <int DC, int KIND>
+static int gpr_gx_launch_kind(const KbwdParams& p, dim3 grid, size_t smem, double* gX, long ldgx, cudaStream_t stream) {
+  static std::atomic<int> smem_state[GPB_MAX_DEVICES];
+  if (int rc = ensure_dynamic_smem(gpr_gx_kernel<DC, KIND>, static_cast<int>(smem), smem_state)) return rc;
+  gpr_gx_kernel<DC, KIND><<<grid, KB_THREADS, smem, stream>>>(p, gX, ldgx);
+  count_launch();
+  GPB_CUDA_CHECK(cudaGetLastError());
+  return GPB_OK;
+}
+
+template <int DC>
+static int gpr_gx_launch_cfg(const KbwdParams& p, double* gX, long ldgx, cudaStream_t stream) {
+  const dim3 grid((p.n1 + KB_COLS - 1) / KB_COLS, (p.D + DC - 1) / DC);
+  const size_t smem = kbwd_smem_bytes(p.D);
+  switch (p.kind) {
+    case KERN_RBF: return gpr_gx_launch_kind<DC, KERN_RBF>(p, grid, smem, gX, ldgx, stream);
+    case KERN_EXP: return gpr_gx_launch_kind<DC, KERN_EXP>(p, grid, smem, gX, ldgx, stream);
+    case KERN_MATERN32: return gpr_gx_launch_kind<DC, KERN_MATERN32>(p, grid, smem, gX, ldgx, stream);
+    case KERN_MATERN52: return gpr_gx_launch_kind<DC, KERN_MATERN52>(p, grid, smem, gX, ldgx, stream);
+    case KERN_PERIODIC: return gpr_gx_launch_kind<DC, KERN_PERIODIC>(p, grid, smem, gX, ldgx, stream);
+    default: return gpr_gx_launch_kind<DC, -1>(p, grid, smem, gX, ldgx, stream);
+  }
+}
+
 int gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* ell, int ell_len,
              const double* sigma2, const double* Kinv, long ldk, const double* kdiag_blocks, const double* a,
              int dy, long lda_a, double* g_ell, double* g_sigma2, double* g_noise, void* workspace,
-             size_t workspace_bytes, cudaStream_t stream) {
+             size_t workspace_bytes, double* gX, long ldgx, cudaStream_t stream) {
   if (kind < 0 || kind > KERN_PERIODIC) return GPB_ERR_BADARG;
   if (!X || !Kinv || !kdiag_blocks || !a || !ell || !g_ell || D <= 0 || n <= 0 || dy <= 0) return GPB_ERR_BADARG;
   if (ell_len != 1 && ell_len != D) return GPB_ERR_BADARG;
   if (kind != KERN_LINEAR && !sigma2) return GPB_ERR_BADARG;
+  if (gX && ldgx < D) return GPB_ERR_BADARG;
   if (D > KB_DMAX) return GPB_ERR_UNSUPPORTED;
   KbwdParams p{};
   p.kind = kind;
@@ -854,7 +1024,10 @@ int gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* el
   if (!workspace || workspace_bytes < gpr_grad_workspace_bytes(n, D)) return GPB_ERR_BADARG;
   p.part_h = static_cast<double*>(workspace);
   p.part_g2 = nullptr;
-  return kbwd_launch<true>(p, ncb, g_ell, g_sigma2, g_noise, nullptr, stream);
+  const KbwdParams px = p;     // kbwd_launch adapts the strips to its path; the input gradient sweeps whole columns
+  if (int rc = kbwd_launch<true>(p, ncb, g_ell, g_sigma2, g_noise, nullptr, stream)) return rc;
+  if (!gX) return GPB_OK;
+  return D <= 8 ? gpr_gx_launch_cfg<8>(px, gX, ldgx, stream) : gpr_gx_launch_cfg<16>(px, gX, ldgx, stream);
 }
 
 }  // namespace gpb

@@ -243,8 +243,11 @@ int gpb_gemm_splitk(int mode, int m, int n, int k_total, int k_per_split, double
  *   are rebuilt by the backward call);  workspace: gpb_kuf_stats_workspace_bytes(m, D, dy, chunk_rows).
  * The backward call reduces the gradient with respect to the panels, dLoss/dKfu_c = Kfu_c R + Y_c W^T with
  * R = dLoss/dPhi + (dLoss/dPhi)^T (M x M, symmetric) and W = dLoss/dpsi (M x dy), against dK/d(ell, sigma2, Z):
- *   g_ell (ell_len), g_sigma2 (1) and gZ (M x D, dense) are OVERWRITTEN with the sums over all chunks. */
-size_t gpb_kuf_stats_workspace_bytes(int m, int D, int dy, int chunk_rows);
+ *   g_ell (ell_len), g_sigma2 (1) and gZ (M x D, dense) are OVERWRITTEN with the sums over all chunks.
+ *   gX (optional, n x D, row stride ldgx >= D): receives dLoss/dX, the gradient with respect to the rows of X (each
+ *   chunk's panel gradient reduced with X and Z exchanged, G_c read transposed); NULL skips it.  A workspace for a call
+ *   with gX is sized by gpb_kuf_stats_workspace_bytes(..., with_gx = 1); with_gx = 0 gives the size without it. */
+size_t gpb_kuf_stats_workspace_bytes(int m, int D, int dy, int chunk_rows, int with_gx);
 int gpb_kuf_stats_fwd(int kind, const double* X, long n, long ldx, const double* Y, int dy, long ldy, const double* Z,
                       int m, long ldz, int D, const double* ell, int ell_len, const double* sigma2, int chunk_rows,
                       double* Phi, long ldphi, double* psi, long ldpsi, double* kfu_cache, long ldcache,
@@ -253,19 +256,22 @@ int gpb_kuf_stats_bwd(int kind, const double* X, long n, long ldx, const double*
                       int m, long ldz, int D, const double* ell, int ell_len, const double* sigma2, int chunk_rows,
                       const double* R, long ldr, const double* W, long ldw, const double* kfu_cache, long ldcache,
                       double* g_ell, double* g_sigma2, double* gZ, void* workspace, size_t workspace_bytes,
-                      void* stream);
+                      void* stream, double* gX, long ldgx);
 
 /* ---- fused GPR gradient ------------------------------------------------------------------------------------
  * Given Kinv in the blocked form left by gpb_potri_lower and a = Ky^-1 (y - m) (n x dy, lda_a), reduce
  *    W = 1/2 (dy * Kinv - a a^T)            (dLoss/dKy, SURVEY 10; gptorch/models/gpr.py:47-67)
  * against dK/d(ell, sigma2) without materialising W or K:  g_ell[d] = sum_ij W_ij dK_ij/d ell_d,
  * g_sigma2 = sum_ij W_ij K_ij / sigma2, g_noise = tr W.  Replaces the autograd backward of
- * kernels.K + _compute_kyy + cholesky + trtrs. */
+ * kernels.K + _compute_kyy + cholesky + trtrs.
+ *   gX (optional, n x D, row stride ldgx >= D): receives dLoss/dX = sum_j 2 W_ij dK_ij/dx_i, the gradient with
+ *   respect to the training inputs (deep kernel learning, learned input warps), from W formed on the fly as above --
+ *   no N x N temporary and no extra workspace.  NULL skips it; the hyper-parameter reduction is the same either way. */
 size_t gpb_gpr_grad_workspace_bytes(int n, int D);
 int gpb_gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* ell, int ell_len,
                  const double* sigma2, const double* Kinv, long ldk, const double* kdiag_blocks,
                  const double* a, int dy, long lda_a, double* g_ell, double* g_sigma2, double* g_noise,
-                 void* workspace, size_t workspace_bytes, void* stream);
+                 void* workspace, size_t workspace_bytes, void* stream, double* gX, long ldgx);
 
 #ifdef __cplusplus
 }
