@@ -620,6 +620,42 @@ class GPRCompositeLogLikFn(Function):
 
 
 # ------------------------------------------------------------------------------------------------------
+# cached GPR posterior: predictive mean and variance, differentiable in the test inputs only
+# ------------------------------------------------------------------------------------------------------
+class GPRPredFn(Function):
+    """(mean [n*, dy], diagonal variance [n*, dy]) of GPR._predict (gptorch/models/gpr.py:88-117) against a cached
+    a = Ky^-1 (y - m(X)) and the full symmetric Ky^-1, for a stationary kernel (the mean function is added outside).
+
+    forward : K* = K(x*, X) (gpb_kern_fwd) ; mean = K* a (gpb_gemv_n) ; Q = K* Ky^-1 (one DMMA GEMM) ;
+              var = sigma2 - rowdot(K*, Q).  Q is kept for the backward pass; K* is not.
+    backward: dLoss/dK*_tj = W_tj = g_mean_t . a_j - 2 g_var_t Q_tj is reduced against dk(x*_t, x_j)/dx*_t on the fly
+              by gpb_pred_gx -- no solve, no [n*, N] panel gradient.  Only x* receives a gradient: X, a, Ky^-1 and the
+              hyper-parameters are constants of the posterior.
+    """
+
+    @staticmethod
+    def forward(ctx, kind, x_new, X, a, Kinv, ell, sigma2):
+        ns, dy = x_new.shape[0], a.shape[1]
+        Ks = nv.kern_fwd(kind, x_new, X, ell, sigma2)
+        mean = nv.gemv_n(Ks, a)
+        Q = nv.gemm(nv.GEMM_NN, Ks, Kinv)
+        var = nv._c(sigma2).reshape(1).repeat(ns)
+        nv.rowdot(Ks, Q, alpha=-1.0, out=var, beta=1.0)
+        ctx.kind = kind
+        ctx.save_for_backward(x_new, X, a, Q, ell, sigma2)
+        return mean, var[:, None].expand(ns, dy).contiguous()
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mean, g_var):
+        x_new, X, a, Q, ell, sigma2 = ctx.saved_tensors
+        gx = None
+        if ctx.needs_input_grad[1]:
+            gx = nv.pred_gx(ctx.kind, x_new, X, ell, sigma2, a, g_mean, g_var.sum(1), Q)
+        return None, gx, None, None, None, None, None
+
+
+# ------------------------------------------------------------------------------------------------------
 # VFE sufficient statistics, streamed over row chunks of X
 # ------------------------------------------------------------------------------------------------------
 def kuu_condition_estimate(L, T, iters=6):

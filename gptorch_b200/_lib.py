@@ -81,6 +81,13 @@ SIGNATURES = {
                              c_void_p, c_void_p, c_long]),
 }
 
+# include/gpb200_posterior.h: entry points of a cached GPR posterior (gpb_version() >= 102), mirrored one to one.
+POSTERIOR_SIGNATURES = {
+    "gpb_pred_gx": (c_int, [c_int, c_void_p, c_int, c_long, c_void_p, c_int, c_long, c_int, c_void_p, c_int, c_void_p,
+                            c_void_p, c_int, c_long, c_void_p, c_long, c_void_p, c_void_p, c_long, c_void_p, c_long,
+                            c_void_p]),
+}
+
 _ERRORS = {-1: "bad argument", -2: "alignment (16-byte base, even leading dimension required)",
            -3: "CUDA runtime error", -4: "CUDA driver / tensor-map error", -5: "unsupported configuration"}
 
@@ -102,7 +109,7 @@ def load():
             "libgpb200.so not found at %s -- build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "or `make -C gptorch_b200/csrc`.  gptorch_b200 has no CPU or PyTorch fallback." % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (restype, argtypes) in SIGNATURES.items():
+    for name, (restype, argtypes) in list(SIGNATURES.items()) + list(POSTERIOR_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here means header and library disagree
         fn.restype = restype
         fn.argtypes = argtypes

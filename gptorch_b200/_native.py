@@ -551,3 +551,24 @@ def gpr_grad(kind, X, ell, sigma2, Kinv, ldk, kd, a, gX=None):
          a.stride(0), ptr(g_ell), ptr(g_sig), ptr(g_noise), ptr(ws), ws.numel() * 8, stream_ptr(),
          ptr(gX), gX.stride(0) if gX is not None else 0)
     return g_ell, g_sig, g_noise
+
+
+# ---------------------------------------------------------------------------------------------- cached GPR posterior
+def pred_gx(kind, Xs, X, ell, sigma2, a, g_mean, g_var, Q):
+    """d loss / d x* (ns x D) for mean = K(x*, X) a and var = sigma2 - rowdot(K(x*, X), Q), given the upstream
+    gradients g_mean (ns x dy) and g_var (ns)."""
+    Xs, X, a, g_mean, Q = _c(Xs), _c(X), _c(a), _c(g_mean), _c(Q)
+    ns, D = Xs.shape
+    ell = _c(ell).reshape(-1)
+    g_var = _c(g_var).reshape(-1)
+    gXs = torch.empty((ns, D), dtype=torch.float64, device=Xs.device)
+    call("gpb_pred_gx", kind, ptr(Xs), ns, _ld(Xs), ptr(X), X.shape[0], _ld(X), D, ptr(ell), ell.numel(),
+         ptr(_c(sigma2).reshape(-1)), ptr(a), a.shape[1], _ld(a), ptr(g_mean), _ld(g_mean), ptr(g_var), ptr(Q), _ld(Q),
+         ptr(gXs), gXs.stride(0), stream_ptr())
+    return gXs
+
+
+def _ld(t):
+    """Leading dimension of a row-major 2-D tensor: the row stride, or the row length for a single row (whose row stride
+    torch leaves arbitrary, e.g. 0 for a broadcast gradient)."""
+    return t.stride(0) if t.shape[0] > 1 else t.shape[1]

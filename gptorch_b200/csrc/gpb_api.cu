@@ -5,6 +5,7 @@
 #include <utility>
 #include <algorithm>
 #include "../../include/gpb200.h"
+#include "../../include/gpb200_posterior.h"
 
 namespace gpb {
 const char* last_error();
@@ -60,6 +61,9 @@ int gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* el
              const double* sigma2, const double* Kinv, long ldk, const double* kdiag_blocks, const double* a,
              int dy, long lda_a, double* g_ell, double* g_sigma2, double* g_noise, void* workspace,
              size_t workspace_bytes, double* gX, long ldgx, cudaStream_t stream);
+int pred_gx(int kind, const double* Xs, int ns, long ldxs, const double* X, int n, long ldx, int D, const double* ell,
+            int ell_len, const double* sigma2, const double* a, int dy, long lda, const double* g_mean, long ldgm,
+            const double* g_var, const double* Q, long ldq, double* gXs, long ldgx, cudaStream_t stream);
 }  // namespace gpb
 
 using namespace gpb;
@@ -136,7 +140,7 @@ static inline int kuf_k_per_split(int rows) {
 #pragma GCC visibility push(default)
 extern "C" {
 
-int gpb_version(void) { return 101; }
+int gpb_version(void) { return 102; }
 const char* gpb_last_error(void) { return last_error(); }
 int gpb_block_size(void) { return NB; }
 long gpb_launch_count(void) { return launch_count(); }
@@ -489,6 +493,14 @@ int gpb_gpr_grad(int kind, const double* X, int n, long ldx, int D, const double
                  size_t workspace_bytes, void* stream, double* gX, long ldgx) {
   return gpr_grad(kind, X, n, ldx, D, ell, ell_len, sigma2, Kinv, ldk, kdiag_blocks, a, dy, lda_a, g_ell, g_sigma2,
                   g_noise, workspace, workspace_bytes, gX, ldgx, S(stream));
+}
+
+int gpb_pred_gx(int kind, const double* Xs, int ns, long ldxs, const double* X, int n, long ldx, int D,
+                const double* ell, int ell_len, const double* sigma2, const double* a, int dy, long lda,
+                const double* g_mean, long ldgm, const double* g_var, const double* Q, long ldq, double* gXs, long ldgx,
+                void* stream) {
+  return pred_gx(kind, Xs, ns, ldxs, X, n, ldx, D, ell, ell_len, sigma2, a, dy, lda, g_mean, ldgm, g_var, Q, ldq, gXs,
+                 ldgx, S(stream));
 }
 
 }  // extern "C"

@@ -1030,4 +1030,189 @@ int gpr_grad(int kind, const double* X, int n, long ldx, int D, const double* el
   return D <= 8 ? gpr_gx_launch_cfg<8>(px, gX, ldgx, stream) : gpr_gx_launch_cfg<16>(px, gX, ldgx, stream);
 }
 
+// ================================================================================================
+// test-input gradient of the cached GPR posterior
+// ================================================================================================
+struct PredGxParams {
+  const double* Xs; int ns; long ldxs;     // test inputs x* (targets of the gradient)
+  const double* X; int n; long ldx;        // training inputs
+  int D;
+  const double* ell; int ell_len;
+  const double* sigma2;
+  const double* a; int dy; long lda;       // a = Ky^-1 (y - m(X)), n x dy
+  const double* gm; long ldgm;             // dLoss/dmean, ns x dy
+  const double* gv;                        // dLoss/dvar, ns
+  const double* Q; long ldq;               // Q = K(x*, X) Ky^-1, ns x n
+  double* gX; long ldgx;
+};
+
+constexpr int PG_QLD = KB_ROWS + 1;   // padded row of the staged Q tile: 17 doubles, conflict-free per half-warp
+
+// With mean = K* a and var = sigma2 - rowdot(K*, Q), dLoss/dK*_tj = W_tj = g_mean_t . a_j - 2 g_var_t Q_tj, and
+//   gX*_t = sum_j W_tj dk(x*_t, x_j)/dx*_t,   dk/dx*_td = sigma2 fac1(r2) (x~_jd - x~_td) / ell_d
+// (the g_ell reduction's fac1, zero below the sqrt clamp as in gpr_gx_kernel).  Same layout as gpr_gx_kernel: one CTA
+// owns 128 test rows (one per thread pair; the two halves take alternate training rows) and one chunk of KB_DC feature
+// dimensions, and sweeps EVERY training row, so each test row's sum is complete inside its CTA and is combined in a
+// fixed order -- no [n*, n] panel gradient, no partials, no atomics, deterministic.  W is formed on the fly from the
+// staged 128 x 16 tile of Q (coalesced rows of 128 bytes) and from g_mean . a staged in chunks of KB_DY outputs.
+template <int KB_DC, int KIND>
+__global__ void __launch_bounds__(KB_THREADS, 2) pred_gx_kernel(const PredGxParams p) {
+  extern __shared__ double kb_smem[];
+  const int D = p.D;
+  double* Xts = kb_smem;                                   // [D][128] test coordinates (scaled)
+  double* Xss = Xts + static_cast<size_t>(D) * KB_COLS;    // [KB_ROWS][D] training coordinates (scaled)
+  double* ellv = Xss + static_cast<size_t>(KB_ROWS) * D;   // [D]
+  double* gmt = ellv + D;                                  // [KB_DY][128] g_mean of the test rows
+  double* as = gmt + KB_COLS * KB_DY;                      // [KB_ROWS][KB_DY]
+  double* Qs = as + KB_ROWS * KB_DY;                       // [128][PG_QLD]
+  double* comb = Qs + KB_COLS * PG_QLD;                    // [2][128]
+
+  const int t = threadIdx.x, c = t & 127, half = t >> 7;
+  const int c0 = blockIdx.x * KB_COLS;
+  const int j = c0 + c;                                    // test row
+  const bool jvalid = j < p.ns;
+  const int d0 = blockIdx.y * KB_DC;
+
+  for (int d = t; d < D; d += KB_THREADS) ellv[d] = p.ell[p.ell_len == 1 ? 0 : d];
+  __syncthreads();
+  for (int idx = t; idx < KB_COLS * D; idx += KB_THREADS) {
+    const int cc = idx / D, d = idx - cc * D;
+    Xts[d * KB_COLS + cc] = (c0 + cc < p.ns) ? p.Xs[static_cast<long>(c0 + cc) * p.ldxs + d] / ellv[d] : 0.0;
+  }
+  const double sig2 = *p.sigma2;
+  const double gv2 = jvalid ? 2.0 * p.gv[j] : 0.0;
+
+  double acc[KB_DC];
+#pragma unroll
+  for (int dd = 0; dd < KB_DC; ++dd) acc[dd] = 0.0;
+
+  const int nrc = (p.n + KB_ROWS - 1) / KB_ROWS;
+  for (int rc = 0; rc < nrc; ++rc) {
+    const int i0 = rc * KB_ROWS;
+    __syncthreads();
+    for (int idx = t; idx < KB_ROWS * D; idx += KB_THREADS) {
+      const int rr = idx / D, d = idx - rr * D;
+      Xss[rr * D + d] = (i0 + rr < p.n) ? p.X[static_cast<long>(i0 + rr) * p.ldx + d] / ellv[d] : 0.0;
+    }
+    for (int idx = t; idx < KB_COLS * KB_ROWS; idx += KB_THREADS) {
+      const int cc = idx / KB_ROWS, k = idx - cc * KB_ROWS;
+      Qs[cc * PG_QLD + k] = (c0 + cc < p.ns && i0 + k < p.n) ? p.Q[static_cast<long>(c0 + cc) * p.ldq + i0 + k] : 0.0;
+    }
+    // gma[rr] = sum_o g_mean[t][o] a[s][o], staged in chunks of KB_DY outputs
+    double hreg[KB_RT];
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) hreg[rr] = 0.0;
+    for (int o0 = 0; o0 < p.dy; o0 += KB_DY) {
+      __syncthreads();
+      for (int idx = t; idx < KB_COLS * KB_DY; idx += KB_THREADS) {
+        const int cc = idx / KB_DY, o = idx - cc * KB_DY;
+        gmt[o * KB_COLS + cc] = (c0 + cc < p.ns && o0 + o < p.dy) ? p.gm[static_cast<long>(c0 + cc) * p.ldgm + o0 + o] : 0.0;
+      }
+      for (int idx = t; idx < KB_ROWS * KB_DY; idx += KB_THREADS) {
+        const int rr = idx / KB_DY, o = idx - rr * KB_DY;
+        as[idx] = (i0 + rr < p.n && o0 + o < p.dy) ? p.a[static_cast<long>(i0 + rr) * p.lda + o0 + o] : 0.0;
+      }
+      __syncthreads();
+#pragma unroll
+      for (int o = 0; o < KB_DY; ++o) {
+        const double gj = gmt[o * KB_COLS + c];
+#pragma unroll
+        for (int rr = 0; rr < KB_RT; ++rr) hreg[rr] += as[(half * KB_RT + rr) * KB_DY + o] * gj;
+      }
+    }
+    __syncthreads();
+
+    double r2[KB_RT];
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) r2[rr] = 0.0;
+    for (int d = 0; d < D; ++d) {
+      const double xt = Xts[d * KB_COLS + c];
+#pragma unroll
+      for (int rr = 0; rr < KB_RT; ++rr) {
+        const double diff = Xss[(half * KB_RT + rr) * D + d] - xt;
+        r2[rr] += diff * diff;
+      }
+    }
+#pragma unroll
+    for (int rr = 0; rr < KB_RT; ++rr) {
+      const int i = i0 + half * KB_RT + rr;
+      double h = 0.0;
+      if (jvalid && i < p.n) {
+        const double w = hreg[rr] - gv2 * Qs[c * PG_QLD + half * KB_RT + rr];
+        double kbase, fac1;
+        kern_base_fac(KIND, r2[rr], kbase, fac1);
+        h = w * fac1 * sig2;
+      }
+      hreg[rr] = h;
+    }
+#pragma unroll
+    for (int dd = 0; dd < KB_DC; ++dd) {
+      const int d = d0 + dd;
+      if (d < D) {
+        const double xt = Xts[d * KB_COLS + c];
+#pragma unroll
+        for (int rr = 0; rr < KB_RT; ++rr) acc[dd] += hreg[rr] * (Xss[(half * KB_RT + rr) * D + d] - xt);
+      }
+    }
+  }
+
+  // the two halves' sums of each test row, in a fixed order; then the 1/ell factor
+#pragma unroll
+  for (int dd = 0; dd < KB_DC; ++dd) {
+    const int d = d0 + dd;
+    if (d >= D) break;  // uniform across the block
+    __syncthreads();
+    comb[half * KB_COLS + c] = acc[dd];
+    __syncthreads();
+    if (half == 0 && jvalid) p.gX[static_cast<long>(j) * p.ldgx + d] = (comb[c] + comb[KB_COLS + c]) / ellv[d];
+  }
+}
+
+static inline size_t pred_gx_smem_bytes(int D) {
+  return (static_cast<size_t>(D) * KB_COLS + static_cast<size_t>(KB_ROWS) * D + D + KB_COLS * KB_DY + KB_ROWS * KB_DY +
+          KB_COLS * PG_QLD + 2 * KB_COLS) * sizeof(double);
+}
+
+template <int DC, int KIND>
+static int pred_gx_launch_kind(const PredGxParams& p, cudaStream_t stream) {
+  static std::atomic<int> smem_state[GPB_MAX_DEVICES];
+  const size_t smem = pred_gx_smem_bytes(p.D);
+  if (int rc = ensure_dynamic_smem(pred_gx_kernel<DC, KIND>, static_cast<int>(smem), smem_state)) return rc;
+  const dim3 grid((p.ns + KB_COLS - 1) / KB_COLS, (p.D + DC - 1) / DC);
+  pred_gx_kernel<DC, KIND><<<grid, KB_THREADS, smem, stream>>>(p);
+  count_launch();
+  GPB_CUDA_CHECK(cudaGetLastError());
+  return GPB_OK;
+}
+
+template <int DC>
+static int pred_gx_launch_cfg(const PredGxParams& p, int kind, cudaStream_t stream) {
+  switch (kind) {
+    case KERN_RBF: return pred_gx_launch_kind<DC, KERN_RBF>(p, stream);
+    case KERN_EXP: return pred_gx_launch_kind<DC, KERN_EXP>(p, stream);
+    case KERN_MATERN32: return pred_gx_launch_kind<DC, KERN_MATERN32>(p, stream);
+    case KERN_MATERN52: return pred_gx_launch_kind<DC, KERN_MATERN52>(p, stream);
+    default: return pred_gx_launch_kind<DC, KERN_PERIODIC>(p, stream);
+  }
+}
+
+int pred_gx(int kind, const double* Xs, int ns, long ldxs, const double* X, int n, long ldx, int D, const double* ell,
+            int ell_len, const double* sigma2, const double* a, int dy, long lda, const double* g_mean, long ldgm,
+            const double* g_var, const double* Q, long ldq, double* gXs, long ldgx, cudaStream_t stream) {
+  if (!kind_has_distance(kind)) return GPB_ERR_BADARG;
+  if (!Xs || !X || !ell || !sigma2 || !a || !g_mean || !g_var || !Q || !gXs) return GPB_ERR_BADARG;
+  if (ns <= 0 || n <= 0 || D <= 0 || dy <= 0 || (ell_len != 1 && ell_len != D)) return GPB_ERR_BADARG;
+  if (ldxs < D || ldx < D || lda < dy || ldgm < dy || ldq < n || ldgx < D) return GPB_ERR_BADARG;
+  if (D > KB_DMAX) return GPB_ERR_UNSUPPORTED;
+  PredGxParams p;
+  p.Xs = Xs; p.ns = ns; p.ldxs = ldxs;
+  p.X = X; p.n = n; p.ldx = ldx;
+  p.D = D; p.ell = ell; p.ell_len = ell_len; p.sigma2 = sigma2;
+  p.a = a; p.dy = dy; p.lda = lda;
+  p.gm = g_mean; p.ldgm = ldgm; p.gv = g_var;
+  p.Q = Q; p.ldq = ldq;
+  p.gX = gXs; p.ldgx = ldgx;
+  return D <= 8 ? pred_gx_launch_cfg<8>(p, kind, stream) : pred_gx_launch_cfg<16>(p, kind, stream);
+}
+
 }  // namespace gpb
