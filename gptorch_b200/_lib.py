@@ -88,6 +88,11 @@ POSTERIOR_SIGNATURES = {
                             c_void_p]),
 }
 
+# include/gpb200_i8mma.h: the switch of the fused int8-sliced engine (gpb_version() >= 103), mirrored one to one.
+I8MMA_SIGNATURES = {
+    "gpb_i8mma_config": (c_int, [c_int]),
+}
+
 _ERRORS = {-1: "bad argument", -2: "alignment (16-byte base, even leading dimension required)",
            -3: "CUDA runtime error", -4: "CUDA driver / tensor-map error", -5: "unsupported configuration"}
 
@@ -109,7 +114,7 @@ def load():
             "libgpb200.so not found at %s -- build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "or `make -C gptorch_b200/csrc`.  gptorch_b200 has no CPU or PyTorch fallback." % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (restype, argtypes) in list(SIGNATURES.items()) + list(POSTERIOR_SIGNATURES.items()):
+    for name, (restype, argtypes) in list(SIGNATURES.items()) + list(POSTERIOR_SIGNATURES.items()) + list(I8MMA_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError here means header and library disagree
         fn.restype = restype
         fn.argtypes = argtypes

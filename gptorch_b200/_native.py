@@ -399,8 +399,9 @@ def gemm(mode, A, B, alpha=1.0, beta=0.0, C=None, lower_only=False, flags=0):
 
 
 def gemm_ozaki_nt(A, B, slices=8, alpha=1.0, beta=0.0, C=None, lower_only=False):
-    """EXPERIMENTAL: C = alpha A B^T + beta C on the INT8 tensor path by integer slicing (gpb_gemm_ozaki_nt); raises
-    NativeLibraryError with status -5 for shapes that path does not take."""
+    """C = alpha A B^T + beta C on the INT8 tensor path by integer slicing (gpb_gemm_ozaki_nt): the fused tcgen05 kernel,
+    or the library engine while ozaki_config() is above 0; raises NativeLibraryError with status -5 for shapes that path
+    does not take."""
     A = _gemm_operand(A)
     B = A if B is None else _gemm_operand(B)
     m, k = A.shape
@@ -418,9 +419,15 @@ def gemm_ozaki_nt(A, B, slices=8, alpha=1.0, beta=0.0, C=None, lower_only=False)
 
 
 def ozaki_config(slices=-1):
-    """Slices used by the blocked Cholesky / inverse for their large products (0 = FP64 DMMA engine, the default).
-    Returns the previous value; slices < 0 only queries."""
+    """Slices of the library (cuBLASLt) engine for the large products of the blocked Cholesky and inverse; 0 = off, the
+    default.  Above 0 it takes precedence over i8mma_config.  Returns the previous value; slices < 0 only queries."""
     return query("gpb_ozaki_config", int(slices))
+
+
+def i8mma_config(slices=-1):
+    """Slices of the fused tcgen05 int8 engine for the large trailing updates of the blocked Cholesky (2..8; 8, the
+    default; 0 = FP64 DMMA engine).  Returns the previous value; slices < 0 only queries."""
+    return query("gpb_i8mma_config", int(slices))
 
 
 def gemv_t(A, Y, out, beta=1.0):

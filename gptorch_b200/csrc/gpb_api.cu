@@ -6,6 +6,7 @@
 #include <algorithm>
 #include "../../include/gpb200.h"
 #include "../../include/gpb200_posterior.h"
+#include "../../include/gpb200_i8mma.h"
 
 namespace gpb {
 const char* last_error();
@@ -17,6 +18,8 @@ int gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long lda, 
                   double* C, long ldc, int lower, int slices, cudaStream_t stream);
 int ozaki_slices();
 void ozaki_set_slices(int s);
+int i8mma_slices();
+void i8mma_set_slices(int s);
 size_t potri_workspace_bytes(int n);
 int potri_lower(double* A, int n, long lda, const double* dinv, double* kdiag_blocks, void* workspace,
                 size_t workspace_bytes, cudaStream_t stream);
@@ -140,7 +143,7 @@ static inline int kuf_k_per_split(int rows) {
 #pragma GCC visibility push(default)
 extern "C" {
 
-int gpb_version(void) { return 102; }
+int gpb_version(void) { return 103; }
 const char* gpb_last_error(void) { return last_error(); }
 int gpb_block_size(void) { return NB; }
 long gpb_launch_count(void) { return launch_count(); }
@@ -252,6 +255,11 @@ int gpb_gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long l
 int gpb_ozaki_config(int slices) {
   const int prev = ozaki_slices();
   if (slices >= 0) ozaki_set_slices(slices);
+  return prev;
+}
+int gpb_i8mma_config(int slices) {
+  const int prev = i8mma_slices();
+  if (slices >= 0) i8mma_set_slices(slices);
   return prev;
 }
 

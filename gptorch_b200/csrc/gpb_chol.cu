@@ -393,11 +393,11 @@ static int get_aux(cudaStream_t caller, AuxStream** out) {
   return GPB_OK;
 }
 
-// EXPERIMENTAL (gpb_ozaki.cu, off unless GPB_OZAKI / gpb_ozaki_config sets a slice count): large trailing updates on the
-// INT8 tensor path.  Shapes that path does not take fall through to the DMMA engine.
+// Large trailing updates on the INT8 tensor path (gpb_ozaki.cu: the fused tcgen05 kernel by default, GPB_I8MMA=0 turns it
+// off).  Shapes that path does not take fall through to the DMMA engine.
 static int syrk_update(CholCtx& c, int r0, int m, int k0, int k) {
   // A[r0:r0+m, r0:r0+m] (lower tiles) -= P P^T with P = A[r0:r0+m, k0:k0+k]
-  if (const int oz = ozaki_slices(); oz > 0 && m >= OZ_MIN_ROWS && k >= OZ_MIN_K) {
+  if (const int oz = sliced_slices(); oz > 0 && m >= OZ_MIN_ROWS && k >= OZ_MIN_K) {
     const double* P = c.A + static_cast<long>(r0) * c.lda + k0;
     const int rc = gemm_ozaki_nt(m, m, k, -1.0, P, c.lda, P, c.lda, 1.0, c.A + static_cast<long>(r0) * c.lda + r0, c.lda, 1,
                                  oz, c.stream);
@@ -429,9 +429,9 @@ static void panel_schedule(int n, std::vector<int>& starts) {
   // trailing updates are short (n = 8192: 512 columns 10.7 ms vs 2048 columns 12.7 ms vs plain recursion 13.4 ms), wide
   // panels once the k-length of the trailing GEMMs dominates (n = 32768: 2048 columns 354 ms, 1024 columns 357 ms)
   int def = n <= 16384 ? 512 : (n <= 24576 ? 1024 : LA_PANEL);
-  // EXPERIMENTAL int8-sliced engine on: its recombination traffic per update is independent of the panel width, so wide panels
-  // pay earlier (n = 16384, 8 slices: 512 columns 49.6 ms, 1024 columns 43.9 ms, 2048 columns 39.5 ms; n = 32768 flat)
-  if (ozaki_slices() > 0 && n >= 12288) def = LA_PANEL;
+  // int8-sliced products: they run the bulk updates so much faster than the panel chain that wide panels pay earlier
+  // (library engine, n = 16384, 8 slices: 512 columns 49.6 ms, 1024 columns 43.9 ms, 2048 columns 39.5 ms; n = 32768 flat)
+  if (sliced_slices() > 0 && n >= 12288) def = LA_PANEL;
   static const int w_env = env_int("GPB_LA_PANEL", 0), first_env = env_int("GPB_LA_FIRST", 0),
                    tail_env = env_int("GPB_LA_TAIL", 0);
   const int w = w_env ? w_env : def, first = first_env ? first_env : w, tail = tail_env ? tail_env : w;
@@ -486,7 +486,7 @@ static int potrf_lookahead(CholCtx& c) {
       g.ax = c0; g.ay = c2;
       g.bx = c0; g.by = c1;
       rc = GPB_ERR_UNSUPPORTED;
-      if (const int oz = ozaki_slices(); oz > 0 && g.M >= OZ_MIN_ROWS && g.N >= OZ_MIN_COLS && g.K >= OZ_MIN_K)
+      if (const int oz = sliced_slices(); oz > 0 && g.M >= OZ_MIN_ROWS && g.N >= OZ_MIN_COLS && g.K >= OZ_MIN_K)
         rc = gemm_ozaki_nt(g.M, g.N, g.K, -1.0, c.A + static_cast<long>(c2) * c.lda + c0, c.lda,
                            c.A + static_cast<long>(c1) * c.lda + c0, c.lda, 1.0, g.C, c.lda, 0, oz, s0);
       if (rc == GPB_ERR_UNSUPPORTED) rc = gemm_launch(GEMM_NT, c.mapA128, c.mapA128, g, s0);
@@ -671,8 +671,8 @@ int trtri_upper(double* A, int n, long lda, const double* dinv, void* workspace,
       g1.batch = batch;
       rc = GPB_ERR_UNSUPPORTED;
       if (const int oz = ozaki_slices(); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
-        // EXPERIMENTAL int8 path: rows [a0, a0 + R) of P^T only involve rows 0 .. a0 + R of T22 and L21; both operands are
-        // stored with the contraction index as the row, so the split transposes them
+        // int8-sliced path (library engine only, see potri_lower): rows [a0, a0 + R) of P^T only involve rows 0 .. a0 + R
+        // of T22 and L21; both operands are stored with the contraction index as the row, so the split transposes them
         rc = GPB_OK;
         for (int pb = 0; pb < batch && rc == GPB_OK; ++pb) {
           const long o2 = off + static_cast<long>(pb) * 2 * s;
@@ -703,7 +703,7 @@ int trtri_upper(double* A, int n, long lda, const double* dinv, void* workspace,
       g2.batch = batch;
       rc = GPB_ERR_UNSUPPORTED;
       if (const int oz = ozaki_slices(); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
-        // EXPERIMENTAL int8 path, per problem and per row strip of T11 (entries from the strip's first column on)
+        // int8-sliced path, per problem and per row strip of T11 (entries from the strip's first column on)
         rc = GPB_OK;
         for (int pb = 0; pb < batch && rc == GPB_OK; ++pb) {
           const long o2 = off + static_cast<long>(pb) * 2 * s;
@@ -737,8 +737,13 @@ int potri_lower(double* A, int n, long lda, const double* dinv, double* kdiag_bl
   rc = make_tmap_f64(&mapA128, A, n, n, lda, 32);
   if (rc) return rc;
   // Kinv = T T^T: strictly-lower blocks in place, diagonal blocks to kdiag_blocks.
+  // The inverse's products take the int8-sliced path only with the library engine switched on (GPB_OZAKI, opt-in), not
+  // with the default fused kernel: Ky^-1 feeds sums that cancel (the GPR gradient's tr(Ky^-1 dK), the predictive
+  // variance), which amplify the products' norm-wise error.  Measured on B200 with 8 slices, inverse products sliced vs
+  // on the DMMA engine: N = 16384 variance gradient 1.4e-7 vs 2.4e-9 from the reference, N = 32768 Ky^-1 (Ky v) - v
+  // 1.5e-8 vs 1.5e-10 -- the factor's sliced updates alone keep both inside the 1e-7 / 1e-8 tolerances.
   if (const int oz = ozaki_slices(); oz > 0 && n >= OZ_MIN_ROWS && (n & 15) == 0) {
-    // EXPERIMENTAL int8 path: row strip [i0, i0 + R) of T only has entries from column i0 on, so its product with the rows
+    // int8-sliced path: row strip [i0, i0 + R) of T only has entries from column i0 on, so its product with the rows
     // 0 .. i0 + R runs over k in [i0, n) -- one independent sliced product per strip, no flop on the zero triangle
     rc = GPB_OK;
     for (int i0 = 0; i0 < n && rc == GPB_OK; i0 += OZ_TRI_STRIP) {

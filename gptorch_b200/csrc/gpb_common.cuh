@@ -145,5 +145,9 @@ __device__ __forceinline__ double block_sum(double v, double* scratch) {
 // Encode a 2-D fp64 row-major tensor map: `rows` x `cols` view at `base` with leading dimension `ld`
 // (elements), box = box_rows x 16 columns (128 bytes, SWIZZLE_128B), out-of-bounds elements read as 0.
 int make_tmap_f64(CUtensorMap* out, const double* base, long rows, long cols, long ld, int box_rows);
+// Encode the int8 slice buffer of the sliced GEMM (`rows` rows of `slices` x k bytes, slice-major inside a row) as a 3-D
+// map (k, slice, row); box = box_rows rows x box_k bytes of ONE slice, swizzled by box_k (32, 64 or 128 bytes), k beyond
+// the slice and rows beyond `rows` read as 0.
+int make_tmap_i8_slices(CUtensorMap* out, const int8_t* base, long rows, int k, int slices, int box_k, int box_rows);
 
 }  // namespace gpb

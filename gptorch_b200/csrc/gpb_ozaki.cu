@@ -1,5 +1,11 @@
-// gpb_ozaki.cu -- EXPERIMENTAL, off by default: FP64-equivalent C = beta C + alpha A B^T on the INT8 tensor path by
-// integer slicing (Ozaki scheme).  DESIGN.md section 8; measurements in profiles/r02_ozaki_*.txt.
+// gpb_ozaki.cu -- FP64-equivalent C = beta C + alpha A B^T on the INT8 tensor path by integer slicing (Ozaki scheme):
+// the split kernels, the driver of both product engines and the library engine.  DESIGN.md section 8; measurements in
+// profiles/r02_ozaki_*.txt and profiles/r05_*.json.
+//
+// Two engines share the split and the workspace.  The default is this library's fused tcgen05 kernel
+// (gpb_ozaki_mma.cu: products and recombination in one launch, GPB_I8MMA / gpb_i8mma_config).  The library engine
+// described below (GPB_OZAKI / gpb_ozaki_config) takes precedence while switched on; it is the bitwise reference of the
+// fused kernel.
 //
 // Every row of A (m x k) and B (n x k), both K-major, is scaled by a power of two 2^-e_i so that |a| <= 1/2 and cut into
 // S signed 7-bit slices, a = 2^e sum_s q_s 2^(-7 (s + 1)), q_s in [-64, 64] (error-free: each remainder is exact in
@@ -13,8 +19,8 @@
 // produced in strips of OZ_STRIP rows; with `lower` only the columns up to the strip's diagonal block are computed.
 //
 // Error model: |dC_ij| <= k 2^(-7 S + 1) max|A_i.| max|B_j.| -- norm-wise like a DGEMM for S = 8 (measured on
-// covariance-conditioned operands: tools/ozaki_probe.py), weaker component-wise, which is why this path is opt-in
-// (GPB_OZAKI=<slices> or gpb_ozaki_config) and the FP64 DMMA engine stays the default.
+// covariance-conditioned operands: tools/ozaki_probe.py), weaker component-wise (DESIGN.md section 8 says why 8 slices
+// are the default for the GPR path's products; GPB_I8MMA=0 returns them to the FP64 DMMA engine).
 #include "gpb_common.cuh"
 #include "gpb_ozaki.cuh"
 #include <cublasLt.h>
@@ -63,6 +69,7 @@ static std::mutex g_oz_mutex;
 static LtApi g_lt;
 static std::map<std::pair<int, cudaStream_t>, OzState> g_oz_state;
 static std::atomic<int> g_oz_slices{-1};   // -1 = read GPB_OZAKI on first use
+static std::atomic<int> g_mma_slices{-1};  // -1 = read GPB_I8MMA on first use
 
 static int lt_load() {
   if (g_lt.status) return g_lt.status > 0 ? GPB_OK : GPB_ERR_UNSUPPORTED;
@@ -319,22 +326,47 @@ int ozaki_slices() {
   return s;
 }
 
+int i8mma_slices() {
+  int s = g_mma_slices.load(std::memory_order_relaxed);
+  if (s < 0) {
+    const char* e = getenv("GPB_I8MMA");
+    s = e && *e ? atoi(e) : OZ_MMA_DEFAULT_SLICES;
+    s = (s < 0 || s == 1 || s > OZ_MMA_MAX_SLICES) ? OZ_MMA_DEFAULT_SLICES : s;
+    g_mma_slices.store(s, std::memory_order_relaxed);
+  }
+  return s;
+}
+
+int sliced_slices() {
+  const int oz = ozaki_slices();
+  return oz > 0 ? oz : i8mma_slices();
+}
+
+// switching a sliced engine off returns the workspaces (hundreds of MB at N = 32768, several GB for the library engine)
+// of the current device
+static void free_workspaces() {
+  std::lock_guard<std::mutex> lock(g_oz_mutex);
+  int dev = -1;
+  if (cudaGetDevice(&dev) != cudaSuccess) return;
+  for (auto& kv : g_oz_state) {
+    if (kv.first.first != dev || !kv.second.ws) continue;
+    cudaDeviceSynchronize();
+    cudaFree(kv.second.ws);
+    kv.second.ws = nullptr;
+    kv.second.ws_bytes = 0;
+  }
+}
+
 void ozaki_set_slices(int s) {
   s = (s < 0 || s > OZ_MAX_SLICES) ? 0 : (s == 1 ? 8 : s);     // 1 = "on" = 8 slices, as for GPB_OZAKI
   g_oz_slices.store(s, std::memory_order_relaxed);
-  if (s == 0) {
-    // switching the path off returns its workspaces (several GB at N = 32768) of the current device
-    std::lock_guard<std::mutex> lock(g_oz_mutex);
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) return;
-    for (auto& kv : g_oz_state) {
-      if (kv.first.first != dev || !kv.second.ws) continue;
-      cudaDeviceSynchronize();
-      cudaFree(kv.second.ws);
-      kv.second.ws = nullptr;
-      kv.second.ws_bytes = 0;
-    }
-  }
+  if (s == 0) free_workspaces();
+}
+
+void i8mma_set_slices(int s) {
+  s = (s == 1 || s > OZ_MMA_MAX_SLICES) ? OZ_MMA_DEFAULT_SLICES : s;
+  g_mma_slices.store(s, std::memory_order_relaxed);
+  if (s == 0) free_workspaces();
 }
 
 int gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long lda, const double* B, long ldb, double beta,
@@ -355,18 +387,24 @@ int gemm_ozaki_nt_ex(const OzEx& x) {
   if (m <= 0 || n <= 0) return GPB_OK;
   if (!A || !B || !C || k <= 0 || lda < (x.a_trans ? m : k) || ldb < (x.b_trans ? n : k) || ldc < n) return GPB_ERR_BADARG;
   if (slices < 2 || slices > OZ_MAX_SLICES) return GPB_ERR_BADARG;
-  // shapes the int8 library path takes (everything else stays on the DMMA engine)
+  // shapes the int8 path takes (everything else stays on the DMMA engine)
   if ((k & 15) || (m & 3) || (n & 3) || (ldc & 1)) return GPB_ERR_UNSUPPORTED;
   if ((x.a_tri && (x.a_col0 & 3)) || (x.b_tri && (x.b_col0 & 3)) || (x.gi0 & 3)) return GPB_ERR_UNSUPPORTED;
   if (static_cast<long long>(k) * slices * 4096 >= (1LL << 31)) return GPB_ERR_UNSUPPORTED;
   if (lower && x.gi0 == 0 && x.Cdiag == nullptr && m != n) return GPB_ERR_BADARG;
+  // the library engine while GPB_OZAKI / gpb_ozaki_config asks for it, this library's fused kernel otherwise
+  const bool native = ozaki_slices() == 0;
+  if (native && slices > OZ_MMA_MAX_SLICES) return GPB_ERR_UNSUPPORTED;
   std::lock_guard<std::mutex> lock(g_oz_mutex);
-  int rc = lt_load();
-  if (rc) return rc;
+  int rc = GPB_OK;
   int dev = 0;
   GPB_CUDA_CHECK(cudaGetDevice(&dev));
   OzState& st = g_oz_state[std::make_pair(dev, stream)];
-  if (!st.handle && g_lt.Create(&st.handle) != CUBLAS_STATUS_SUCCESS) return GPB_ERR_UNSUPPORTED;
+  if (!native) {
+    rc = lt_load();
+    if (rc) return rc;
+    if (!st.handle && g_lt.Create(&st.handle) != CUBLAS_STATUS_SUCCESS) return GPB_ERR_UNSUPPORTED;
+  }
 
   const int S = slices;
   const bool same = (A == B && lda == ldb && m == n && !x.a_trans && !x.b_trans && x.a_tri == x.b_tri &&
@@ -375,14 +413,20 @@ int gemm_ozaki_nt_ex(const OzEx& x) {
   const int strip = OZ_STRIP;
   const long ldp = (static_cast<long>(n) + 15) & ~15L;
   const long plane = static_cast<long>(strip) * ldp;
+  // workspace: the slices and the scales; the library engine adds its int32 class planes and its own workspace.  The
+  // fused kernel reads B in the forward slice order, so for A A^T it reads A's slices twice instead of a second copy.
   size_t off = 0;
   const size_t o_a8 = off;   off += oz_align(static_cast<size_t>(m) * ld8);
-  const size_t o_b8 = off;   off += oz_align(static_cast<size_t>(n) * ld8);
+  const size_t o_b8 = off;   off += (native && same) ? 0 : oz_align(static_cast<size_t>(n) * ld8);
   const size_t o_sa = off;   off += oz_align(static_cast<size_t>(m) * sizeof(double));
   const size_t o_sb = off;   off += oz_align(static_cast<size_t>(n) * sizeof(double));
-  const size_t o_p = off;    off += oz_align(static_cast<size_t>(S) * plane * sizeof(int32_t));
-  const size_t o_lt = off;   off += OZ_LT_WORKSPACE;
+  const size_t o_p = off;    off += native ? 0 : oz_align(static_cast<size_t>(S) * plane * sizeof(int32_t));
+  const size_t o_lt = off;   off += native ? 0 : OZ_LT_WORKSPACE;
   if (off > st.ws_bytes) {
+    // a stream being captured into a CUDA graph cannot allocate: such products stay on the DMMA engine
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    GPB_CUDA_CHECK(cudaStreamIsCapturing(stream, &cap));
+    if (cap != cudaStreamCaptureStatusNone) return GPB_ERR_UNSUPPORTED;
     if (st.ws) {
       GPB_CUDA_CHECK(cudaStreamSynchronize(stream));
       GPB_CUDA_CHECK(cudaFree(st.ws));
@@ -393,11 +437,12 @@ int gemm_ozaki_nt_ex(const OzEx& x) {
     st.ws_bytes = off;
   }
   int8_t* a8 = reinterpret_cast<int8_t*>(st.ws + o_a8);
-  int8_t* b8 = reinterpret_cast<int8_t*>(st.ws + o_b8);
+  int8_t* b8 = (native && same) ? a8 : reinterpret_cast<int8_t*>(st.ws + o_b8);
   double* sa = reinterpret_cast<double*>(st.ws + o_sa);
   double* sb = same ? sa : reinterpret_cast<double*>(st.ws + o_sb);
-  int32_t* P = reinterpret_cast<int32_t*>(st.ws + o_p);
-  void* lt_ws = st.ws + o_lt;
+  // B's slices: forward order for the fused kernel, reverse order for the library's concatenated-k products
+  int8_t* b_fwd = native ? b8 : nullptr;
+  int8_t* b_rev = native ? nullptr : b8;
 
   if (x.a_trans) {
     oz_colmax_kernel<<<(m + 31) / 32, 256, 0, stream>>>(A, lda, k, m, sa, x.a_tri, x.a_row0, x.a_col0);
@@ -405,20 +450,25 @@ int gemm_ozaki_nt_ex(const OzEx& x) {
                                                                                x.a_row0, x.a_col0);
     count_launch(2);
   } else {
-    oz_split_kernel<<<m, 256, 0, stream>>>(A, lda, k, S, a8, same ? b8 : nullptr, ld8, sa, x.a_tri, x.a_row0, x.a_col0);
+    oz_split_kernel<<<m, 256, 0, stream>>>(A, lda, k, S, a8, (same && !native) ? b8 : nullptr, ld8, sa, x.a_tri, x.a_row0,
+                                           x.a_col0);
     count_launch();
   }
   if (x.b_trans) {
     oz_colmax_kernel<<<(n + 31) / 32, 256, 0, stream>>>(B, ldb, k, n, sb, x.b_tri, x.b_row0, x.b_col0);
-    oz_split_t_kernel<<<dim3((n + 31) / 32, (k + 127) / 128), 256, 0, stream>>>(B, ldb, k, n, S, nullptr, b8, ld8, sb, x.b_tri,
+    oz_split_t_kernel<<<dim3((n + 31) / 32, (k + 127) / 128), 256, 0, stream>>>(B, ldb, k, n, S, b_fwd, b_rev, ld8, sb, x.b_tri,
                                                                                x.b_row0, x.b_col0);
     count_launch(2);
   } else if (!same) {
-    oz_split_kernel<<<n, 256, 0, stream>>>(B, ldb, k, S, nullptr, b8, ld8, sb, x.b_tri, x.b_row0, x.b_col0);
+    oz_split_kernel<<<n, 256, 0, stream>>>(B, ldb, k, S, b_fwd, b_rev, ld8, sb, x.b_tri, x.b_row0, x.b_col0);
     count_launch();
   }
   GPB_CUDA_CHECK(cudaGetLastError());
 
+  if (native) return ozaki_mma_launch(x, a8, b8, sa, sb);
+
+  void* lt_ws = st.ws + o_lt;
+  int32_t* P = reinterpret_cast<int32_t*>(st.ws + o_p);
   for (int i0 = 0; i0 < m; i0 += strip) {
     const int rows = std::min(strip, m - i0);
     int cols = n;

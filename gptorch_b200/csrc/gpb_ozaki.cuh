@@ -1,4 +1,4 @@
-// gpb_ozaki.cuh -- internal interface of the EXPERIMENTAL int8-sliced GEMM (gpb_ozaki.cu).
+// gpb_ozaki.cuh -- internal interface of the int8-sliced GEMM (gpb_ozaki.cu, gpb_ozaki_mma.cu).
 #pragma once
 #include "gpb_common.cuh"
 
@@ -22,14 +22,24 @@ struct OzEx {
   cudaStream_t stream = nullptr;
 };
 
-// C = beta C + alpha A B^T on the INT8 tensor path; GPB_ERR_UNSUPPORTED for shapes it does not take (callers fall back to
-// the FP64 DMMA engine).
+// C = beta C + alpha A B^T on the INT8 tensor path; GPB_ERR_UNSUPPORTED for shapes it does not take (callers use the FP64
+// DMMA engine for those).
 int gemm_ozaki_nt_ex(const OzEx& x);
 int gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long lda, const double* B, long ldb, double beta,
                   double* C, long ldc, int lower, int slices, cudaStream_t stream);
-// slices configured for the blocked factorisations (0 = off, the default; GPB_OZAKI / gpb_ozaki_config)
+// Engines.  GPB_OZAKI / gpb_ozaki_config: slices of the library engine (cuBLASLt int8 products, 0 = off, the default).
+// GPB_I8MMA / gpb_i8mma_config: slices of the fused tcgen05 kernel (gpb_ozaki_mma.cu; 8 by default, 0 = FP64 DMMA).
+// gemm_ozaki_nt_ex runs the library engine while ozaki_slices() > 0 and the fused kernel otherwise; the Cholesky's
+// updates use sliced_slices() = ozaki_slices() if that is > 0, else i8mma_slices(); the inverse's use ozaki_slices().
 int ozaki_slices();
 void ozaki_set_slices(int s);
+int i8mma_slices();
+void i8mma_set_slices(int s);
+int sliced_slices();
+constexpr int OZ_MMA_MAX_SLICES = 8, OZ_MMA_DEFAULT_SLICES = 8;
+// The fused product (gpb_ozaki_mma.cu) on slices already split by gemm_ozaki_nt_ex: a8 (m rows) and b8 (n rows), both in
+// forward slice order with row pitch slices * k bytes, row scales sa / sb.
+int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const double* sa, const double* sb);
 // thresholds of the hooks in gpb_chol.cu
 constexpr int OZ_MIN_ROWS = 4096, OZ_MIN_COLS = 1024, OZ_MIN_K = 512, OZ_TRI_STRIP = 2048, OZ_TRTRI_MIN_S = 4096;
 

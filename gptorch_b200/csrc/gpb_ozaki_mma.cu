@@ -1,0 +1,302 @@
+// gpb_ozaki_mma.cu -- the int8-sliced FP64-equivalent product C = beta C + alpha A B^T (DESIGN.md section 8) as ONE
+// tcgen05 kernel: all weight-class sums of a 128 x 64 output tile accumulate in tensor memory, and the epilogue
+// recombines them in fp64.  Operands are the slice buffers of oz_split_kernel / oz_split_t_kernel (gpb_ozaki.cu), both
+// in the forward layout (slice s of a row at byte offset s k), with one power-of-two scale per row.
+//
+// Class u = s + t collects the products Q^A_s (Q^B_t)^T.  The B slices of one k-chunk lie in shared memory one after the
+// other (slice-major, 64 rows each), so A_s times B slices t0 .. t0 + nt - 1 is a single MMA of N = 64 nt whose output
+// columns are exactly the accumulators of the classes s + t0 .. s + t0 + nt - 1 (class u at TMEM columns 64 u .. 64 u + 63).
+// Classes u >= S are never formed.  For S = 8 one k-step of 32 bytes is 12 MMAs (N <= 256) instead of 36 of N = 64, and
+// reads A once per MMA: 120 KB of shared memory per 9.4 M MAC, inside the 128 B/clk an SM can deliver.
+//
+// The int32 class sums are exact ((u + 1) k 4096 < 2^31, checked by the driver), and the epilogue runs the operation
+// sequence of oz_recombine_kernel (Horner from class S-1 down, then (alpha sa_i 2^-14) sb_j t, then beta C + val), so the
+// result is bitwise the one of the unfused library engine.
+//
+// Roles (192 threads): warp 0 issues the TMA loads into a ring of stages, warp 1 allocates TMEM and one lane issues the
+// MMAs (tcgen05.commit releases each stage and finally signals the epilogue), warps 2-5 read the class planes with
+// tcgen05.ld (warp w owns TMEM lanes 32 (w % 4) ..) and write C.
+#include "gpb_common.cuh"
+#include "gpb_ozaki.cuh"
+#include <algorithm>
+
+namespace gpb {
+
+namespace {
+
+constexpr int I8_BM = 128, I8_BN = 64;
+constexpr int I8_CH = 64;                          // k bytes per stage and slice (SWIZZLE_64B rows)
+constexpr int I8_RING_BYTES = 192 * 1024;          // shared memory given to the stage ring
+constexpr int I8_THREADS = 192;
+constexpr int I8_GROUP = 16;                       // tile rows visited together (their A rows stay in L2)
+
+struct I8Params {
+  int m, n, k;
+  double alpha, beta;
+  const double* sa;
+  const double* sb;
+  double* C;
+  long ldc;
+  int lower, gi0;
+  double* Cdiag;
+  int a_trans, a_tri, a_row0, a_col0;
+  int b_trans, b_tri, b_row0, b_col0;
+  int tiles_m, tiles_n;
+};
+
+template <int S>
+struct I8Cfg {
+  static constexpr int A_BYTES = S * I8_BM * I8_CH;
+  static constexpr int B_BYTES = S * I8_BN * I8_CH;
+  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
+  static constexpr int STAGES = std::min(8, I8_RING_BYTES / STAGE_BYTES);
+  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 256;
+  static constexpr int TMEM_COLS = S * I8_BN <= 256 ? 256 : 512;
+};
+
+__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map, int x, int y, int z, uint64_t* bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst),
+      "l"(map), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar))
+      : "memory");
+}
+
+// K-major operand tile with 64-byte rows and the 64-byte swizzle: 8-row groups 512 bytes apart (SBO), LBO unused.
+__device__ __forceinline__ uint64_t smem_desc(uint32_t addr) {
+  return static_cast<uint64_t>((addr & 0x3FFFFu) >> 4) | (static_cast<uint64_t>(1) << 16) |
+         (static_cast<uint64_t>((8 * I8_CH) >> 4) << 32) | (static_cast<uint64_t>(1) << 46) | (static_cast<uint64_t>(4) << 61);
+}
+
+// kind::i8 instruction descriptor: s32 accumulator, signed A and B, both K-major, M = 128.
+__host__ __device__ constexpr uint32_t i8_idesc(int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(I8_BM >> 4) << 24);
+}
+
+__device__ __forceinline__ void mma_i8(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
+  asm volatile(
+      "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc));
+}
+
+__device__ __forceinline__ void mma_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+
+__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, uint32_t (&v)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+               : "r"(taddr));
+}
+
+template <int S>
+__global__ void __launch_bounds__(I8_THREADS, 1)
+oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const I8Params p) {
+  using Cfg = I8Cfg<S>;
+  constexpr int STAGES = Cfg::STAGES;
+
+  // ---- tile: groups of I8_GROUP tile rows, column by column inside a group --------------------------------------
+  int tm, tn;
+  {
+    const int t = blockIdx.x;
+    const int per_group = I8_GROUP * p.tiles_n;
+    const int g = t / per_group;
+    const int first = g * I8_GROUP;
+    const int rows = min(I8_GROUP, p.tiles_m - first);
+    const int l = t - g * per_group;
+    tm = first + l % rows;
+    tn = l / rows;
+  }
+  const int m0 = tm * I8_BM, n0 = tn * I8_BN;
+  const int m_last = min(m0 + I8_BM, p.m) - 1, n_last = min(n0 + I8_BN, p.n) - 1;
+  if (p.lower && (n0 >> 7) > ((p.gi0 + m_last) >> 7)) return;          // every column right of every row's diagonal block
+
+  // ---- k range: the triangular-by-blocks operands are zero outside it (the split wrote zeros there) -------------
+  int k_lo = 0, k_hi = p.k;
+  if (p.a_tri) {
+    if (p.a_trans) k_hi = min(k_hi, ((p.a_col0 + m_last) / NB + 1) * NB - p.a_row0);
+    else k_lo = max(k_lo, ((p.a_row0 + m0) / NB) * NB - p.a_col0);
+  }
+  if (p.b_tri) {
+    if (p.b_trans) k_hi = min(k_hi, ((p.b_col0 + n_last) / NB + 1) * NB - p.b_row0);
+    else k_lo = max(k_lo, ((p.b_row0 + n0) / NB) * NB - p.b_col0);
+  }
+  k_lo &= ~(I8_CH - 1);
+  const int nk = k_hi > k_lo ? (k_hi - k_lo + I8_CH - 1) / I8_CH : 0;
+
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_al + STAGES * Cfg::STAGE_BYTES);
+  uint64_t* empty_bar = full_bar + STAGES;
+  uint64_t* acc_bar = empty_bar + STAGES;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_bar + 1);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(&full_bar[s], 1);
+      mbar_init(&empty_bar[s], 1);
+    }
+    mbar_init(acc_bar, 1);
+    mbar_fence_init();
+  }
+  if (warp == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                 "r"(Cfg::TMEM_COLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  const uint32_t tmem = *tmem_slot;
+
+  if (warp == 0) {
+    // =============================== TMA producer ==============================================
+    if (lane == 0) {
+      tma_prefetch_desc(&mapA);
+      tma_prefetch_desc(&mapB);
+      for (int it = 0; it < nk; ++it) {
+        const int s = it % STAGES;
+        mbar_wait(&empty_bar[s], ((it / STAGES) & 1) ^ 1u);
+        mbar_expect_tx(&full_bar[s], Cfg::STAGE_BYTES);
+        const uint32_t a_dst = smem_base + s * Cfg::STAGE_BYTES, b_dst = a_dst + Cfg::A_BYTES;
+        const int kx = k_lo + it * I8_CH;
+#pragma unroll
+        for (int q = 0; q < S; ++q) tma_load_3d(a_dst + q * (I8_BM * I8_CH), &mapA, kx, q, m0, &full_bar[s]);
+#pragma unroll
+        for (int q = 0; q < S; ++q) tma_load_3d(b_dst + q * (I8_BN * I8_CH), &mapB, kx, q, n0, &full_bar[s]);
+      }
+    }
+  } else if (warp == 1) {
+    // =============================== MMA issue ================================================
+    if (lane == 0 && nk > 0) {
+      for (int it = 0; it < nk; ++it) {
+        const int s = it % STAGES;
+        mbar_wait(&full_bar[s], (it / STAGES) & 1);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        const uint32_t a_base = smem_base + s * Cfg::STAGE_BYTES, b_base = a_base + Cfg::A_BYTES;
+#pragma unroll
+        for (int kk = 0; kk < I8_CH / 32; ++kk) {
+#pragma unroll
+          for (int sa = 0; sa < S; ++sa) {
+#pragma unroll
+            for (int t0 = 0; t0 < S - sa; t0 += 4) {
+              const int nt = min(4, S - sa - t0);
+              const uint64_t ad = smem_desc(a_base + sa * (I8_BM * I8_CH) + kk * 32);
+              const uint64_t bd = smem_desc(b_base + t0 * (I8_BN * I8_CH) + kk * 32);
+              const uint32_t acc = (it > 0 || kk > 0 || sa > 0) ? 1u : 0u;   // sa = 0 covers every class first
+              mma_i8(tmem + static_cast<uint32_t>((sa + t0) * I8_BN), ad, bd, i8_idesc(nt * I8_BN), acc);
+            }
+          }
+        }
+        mma_commit(&empty_bar[s]);
+      }
+      mma_commit(acc_bar);
+    }
+  } else {
+    // =============================== epilogue =================================================
+    const int quarter = warp & 3;
+    const int i = m0 + 32 * quarter + lane;
+    const bool row_ok = i < p.m;
+    const uint32_t t_row = tmem + (static_cast<uint32_t>(32 * quarter) << 16);
+    const int gi = p.gi0 + i;
+    // where the 8 columns from n0 + c0 go (nullptr: not stored).  They lie in one 128-block: gpb_potri_lower's diagonal
+    // blocks go to Cdiag ([row][NB]), the blocks right of the diagonal nowhere.
+    auto dest = [&](int c0) -> double* {
+      const int j = n0 + c0;
+      if (!row_ok || j >= p.n || (p.lower && (j >> 7) > (gi >> 7))) return nullptr;
+      if (p.Cdiag != nullptr && (j >> 7) == (gi >> 7)) return p.Cdiag + static_cast<long>(gi) * NB + (j & (NB - 1));
+      return p.C + static_cast<long>(i) * p.ldc + j;
+    };
+    if (nk > 0) {
+      mbar_wait(acc_bar, 0);
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    }
+    const double down = 1.0 / static_cast<double>(1 << 7);
+    const double si = row_ok ? p.alpha * p.sa[i] * (down * down) : 0.0;
+#pragma unroll 1
+    for (int c0 = 0; c0 < I8_BN; c0 += 8) {
+      uint32_t v[S][8];
+      __syncwarp();
+      if (nk > 0) {
+#pragma unroll
+        for (int u = 0; u < S; ++u) tmem_ld_x8(t_row + static_cast<uint32_t>(u * I8_BN + c0), v[u]);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      } else {
+#pragma unroll
+        for (int u = 0; u < S; ++u)
+#pragma unroll
+          for (int q = 0; q < 8; ++q) v[u][q] = 0u;
+      }
+      const int j = n0 + c0;
+      if (double* c = dest(c0)) {
+        double t[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) t[q] = 0.0;
+#pragma unroll
+        for (int u = S - 1; u >= 0; --u)                              // Horner from the smallest weight class up
+#pragma unroll
+          for (int q = 0; q < 8; ++q) t[q] = t[q] * down + static_cast<double>(static_cast<int32_t>(v[u][q]));
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          if (j + q < p.n) {
+            const double val = (si * p.sb[j + q]) * t[q];
+            c[q] = p.beta == 0.0 ? val : p.beta * c[q] + val;
+          }
+        }
+      }
+    }
+  }
+
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == 1) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(Cfg::TMEM_COLS));
+  }
+}
+
+template <int S>
+int launch_s(const CUtensorMap& mapA, const CUtensorMap& mapB, const I8Params& p, cudaStream_t stream) {
+  static std::atomic<int> smem_state[GPB_MAX_DEVICES];
+  if (int rc = ensure_dynamic_smem(oz_mma_kernel<S>, I8Cfg<S>::SMEM_BYTES, smem_state)) return rc;
+  const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
+  oz_mma_kernel<S><<<static_cast<unsigned>(tiles), I8_THREADS, I8Cfg<S>::SMEM_BYTES, stream>>>(mapA, mapB, p);
+  count_launch();
+  GPB_CUDA_CHECK(cudaGetLastError());
+  return GPB_OK;
+}
+
+}  // namespace
+
+int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const double* sa, const double* sb) {
+  const int S = x.slices;
+  CUtensorMap mapA, mapB;
+  int rc = make_tmap_i8_slices(&mapA, a8, x.m, x.k, S, I8_CH, I8_BM);
+  if (rc) return rc;
+  rc = make_tmap_i8_slices(&mapB, b8, x.n, x.k, S, I8_CH, I8_BN);
+  if (rc) return rc;
+  I8Params p;
+  p.m = x.m; p.n = x.n; p.k = x.k;
+  p.alpha = x.alpha; p.beta = x.beta;
+  p.sa = sa; p.sb = sb;
+  p.C = x.C; p.ldc = x.ldc;
+  p.lower = x.lower; p.gi0 = x.gi0; p.Cdiag = x.Cdiag;
+  p.a_trans = x.a_trans; p.a_tri = x.a_tri; p.a_row0 = x.a_row0; p.a_col0 = x.a_col0;
+  p.b_trans = x.b_trans; p.b_tri = x.b_tri; p.b_row0 = x.b_row0; p.b_col0 = x.b_col0;
+  p.tiles_m = (x.m + I8_BM - 1) / I8_BM;
+  p.tiles_n = (x.n + I8_BN - 1) / I8_BN;
+  switch (S) {
+    case 2: return launch_s<2>(mapA, mapB, p, x.stream);
+    case 3: return launch_s<3>(mapA, mapB, p, x.stream);
+    case 4: return launch_s<4>(mapA, mapB, p, x.stream);
+    case 5: return launch_s<5>(mapA, mapB, p, x.stream);
+    case 6: return launch_s<6>(mapA, mapB, p, x.stream);
+    case 7: return launch_s<7>(mapA, mapB, p, x.stream);
+    case 8: return launch_s<8>(mapA, mapB, p, x.stream);
+  }
+  return GPB_ERR_UNSUPPORTED;
+}
+
+}  // namespace gpb

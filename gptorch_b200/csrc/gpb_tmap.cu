@@ -56,4 +56,27 @@ int make_tmap_f64(CUtensorMap* out, const double* base, long rows, long cols, lo
   return GPB_OK;
 }
 
+int make_tmap_i8_slices(CUtensorMap* out, const int8_t* base, long rows, int k, int slices, int box_k, int box_rows) {
+  auto fn = get_encode_fn();
+  if (!fn) { set_last_error_msg("cuTensorMapEncodeTiled entry point unavailable"); return GPB_ERR_DRIVER; }
+  if ((reinterpret_cast<uintptr_t>(base) & 15) || (k & 15) || rows <= 0 || k <= 0 || slices <= 0) {
+    set_last_error_msg("int8 slice tensor map: base must be 16-byte aligned and k a multiple of 16");
+    return GPB_ERR_ALIGN;
+  }
+  cuuint64_t gdim[3] = {static_cast<cuuint64_t>(k), static_cast<cuuint64_t>(slices), static_cast<cuuint64_t>(rows)};
+  cuuint64_t gstr[2] = {static_cast<cuuint64_t>(k), static_cast<cuuint64_t>(k) * slices};
+  cuuint32_t box[3] = {static_cast<cuuint32_t>(box_k), 1u, static_cast<cuuint32_t>(box_rows)};
+  cuuint32_t estr[3] = {1u, 1u, 1u};
+  const CUtensorMapSwizzle swz = box_k == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                 : box_k == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
+  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<int8_t*>(base), gdim, gstr, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled (int8) failed with CUresult %d (rows=%ld k=%d S=%d)",
+             static_cast<int>(r), rows, k, slices);
+    return GPB_ERR_DRIVER;
+  }
+  return GPB_OK;
+}
+
 }  // namespace gpb

@@ -47,3 +47,12 @@ vfe_phi_cond_max = 2.0e5
 # panel product (3 B M^2 flop per loss+grad instead of 6 B M^2) under the same conditioning gate as the VFE Phi form, for
 # batches of at least 16 M rows with the Gaussian likelihood.  False = the reference's order; True = always.
 svgp_quadratic_form = "auto"
+
+
+def int8_sliced_products(slices=None):
+    """Slices of the FP64-equivalent int8 products that run the large O(N^3) trailing updates of the Cholesky factor
+    (DESIGN.md section 8; the inverse stays on the FP64 DMMA engine): 8 by default, 2..8 allowed, 0 = the FP64 DMMA
+    engine.  With an argument it sets the value for the process (and returns the previous one); without, it only
+    queries.  The environment variable GPB_I8MMA sets the initial value."""
+    from . import _native
+    return _native.i8mma_config(-1 if slices is None else int(slices))
