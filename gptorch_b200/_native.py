@@ -426,7 +426,8 @@ def ozaki_config(slices=-1):
 
 def i8mma_config(slices=-1):
     """Slices of the fused tcgen05 int8 engine for the large trailing updates of the blocked Cholesky (2..8; 8, the
-    default; 0 = FP64 DMMA engine).  Returns the previous value; slices < 0 only queries."""
+    default; 0 = FP64 DMMA engine for the factor and the inverse).  While it is above 0 the blocked inverse's products
+    run on the same engine at a fixed 9 slices.  Returns the previous value; slices < 0 only queries."""
     return query("gpb_i8mma_config", int(slices))
 
 

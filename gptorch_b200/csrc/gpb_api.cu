@@ -1,5 +1,6 @@
 // gpb_api.cu -- the extern "C" boundary of libgpb200.so (declared in include/gpb200.h).
 #include "gpb_gemm.cuh"
+#include "gpb_ozaki.cuh"
 #include <map>
 #include <mutex>
 #include <utility>
@@ -143,7 +144,7 @@ static inline int kuf_k_per_split(int rows) {
 #pragma GCC visibility push(default)
 extern "C" {
 
-int gpb_version(void) { return 103; }
+int gpb_version(void) { return 104; }
 const char* gpb_last_error(void) { return last_error(); }
 int gpb_block_size(void) { return NB; }
 long gpb_launch_count(void) { return launch_count(); }
@@ -250,6 +251,9 @@ int gpb_gemv_t(const double* A, long rows, int cols, long lda, const double* Y, 
 
 int gpb_gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long lda, const double* B, long ldb, double beta,
                       double* C, long ldc, int lower, int slices, void* stream) {
+  // on the fused engine the public entry takes the slice counts gpb_i8mma_config takes; more (the blocked inverse's
+  // products, in narrower tiles) are internal
+  if (ozaki_slices() == 0 && slices > OZ_MMA_MAX_SLICES && slices <= OZ_MMA_MAX_TILE_SLICES) return GPB_ERR_UNSUPPORTED;
   return gemm_ozaki_nt(m, n, k, alpha, A, lda, B, ldb, beta, C, ldc, lower, slices, S(stream));
 }
 int gpb_ozaki_config(int slices) {

@@ -670,8 +670,8 @@ int trtri_upper(double* A, int n, long lda, const double* dinv, void* workspace,
       g1.flags = GF_KHI_M;
       g1.batch = batch;
       rc = GPB_ERR_UNSUPPORTED;
-      if (const int oz = ozaki_slices(); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
-        // int8-sliced path (library engine only, see potri_lower): rows [a0, a0 + R) of P^T only involve rows 0 .. a0 + R
+      if (const int oz = inverse_slices(n); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
+        // int8-sliced path (inverse_slices, see potri_lower): rows [a0, a0 + R) of P^T only involve rows 0 .. a0 + R
         // of T22 and L21; both operands are stored with the contraction index as the row, so the split transposes them
         rc = GPB_OK;
         for (int pb = 0; pb < batch && rc == GPB_OK; ++pb) {
@@ -702,7 +702,7 @@ int trtri_upper(double* A, int n, long lda, const double* dinv, void* workspace,
       g2.flags = GF_KLO_M;
       g2.batch = batch;
       rc = GPB_ERR_UNSUPPORTED;
-      if (const int oz = ozaki_slices(); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
+      if (const int oz = inverse_slices(n); oz > 0 && pass == 0 && s >= OZ_TRTRI_MIN_S) {
         // int8-sliced path, per problem and per row strip of T11 (entries from the strip's first column on)
         rc = GPB_OK;
         for (int pb = 0; pb < batch && rc == GPB_OK; ++pb) {
@@ -737,12 +737,12 @@ int potri_lower(double* A, int n, long lda, const double* dinv, double* kdiag_bl
   rc = make_tmap_f64(&mapA128, A, n, n, lda, 32);
   if (rc) return rc;
   // Kinv = T T^T: strictly-lower blocks in place, diagonal blocks to kdiag_blocks.
-  // The inverse's products take the int8-sliced path only with the library engine switched on (GPB_OZAKI, opt-in), not
-  // with the default fused kernel: Ky^-1 feeds sums that cancel (the GPR gradient's tr(Ky^-1 dK), the predictive
-  // variance), which amplify the products' norm-wise error.  Measured on B200 with 8 slices, inverse products sliced vs
-  // on the DMMA engine: N = 16384 variance gradient 1.4e-7 vs 2.4e-9 from the reference, N = 32768 Ky^-1 (Ky v) - v
-  // 1.5e-8 vs 1.5e-10 -- the factor's sliced updates alone keep both inside the 1e-7 / 1e-8 tolerances.
-  if (const int oz = ozaki_slices(); oz > 0 && n >= OZ_MIN_ROWS && (n & 15) == 0) {
+  // The inverse's products (the two trtri_upper hooks and this one) are int8-sliced at inverse_slices(n): 9 slices on
+  // the default fused engine, one more than the factor's.  Ky^-1 feeds sums that cancel (the GPR gradient's
+  // tr(Ky^-1 dK), the predictive variance), which amplify the products' norm-wise error.  Measured on B200 with the
+  // inverse sliced at 8: N = 16384 variance gradient 1.4e-7 from the reference (tolerance 1e-7), N = 32768
+  // Ky^-1 (Ky v) - v 1.5e-8 (tolerance 1e-8); at 9 slices 6e-10 and 1.3e-10 (DESIGN.md section 8).
+  if (const int oz = inverse_slices(n); oz > 0 && n >= OZ_MIN_ROWS) {
     // int8-sliced path: row strip [i0, i0 + R) of T only has entries from column i0 on, so its product with the rows
     // 0 .. i0 + R runs over k in [i0, n) -- one independent sliced product per strip, no flop on the zero triangle
     rc = GPB_OK;

@@ -342,6 +342,13 @@ int sliced_slices() {
   return oz > 0 ? oz : i8mma_slices();
 }
 
+int inverse_slices(int n) {
+  if (n & 15) return 0;
+  const int oz = ozaki_slices();
+  if (oz > 0) return oz;
+  return i8mma_slices() > 0 ? OZ_INV_SLICES : 0;
+}
+
 // switching a sliced engine off returns the workspaces (hundreds of MB at N = 32768, several GB for the library engine)
 // of the current device
 static void free_workspaces() {
@@ -394,7 +401,6 @@ int gemm_ozaki_nt_ex(const OzEx& x) {
   if (lower && x.gi0 == 0 && x.Cdiag == nullptr && m != n) return GPB_ERR_BADARG;
   // the library engine while GPB_OZAKI / gpb_ozaki_config asks for it, this library's fused kernel otherwise
   const bool native = ozaki_slices() == 0;
-  if (native && slices > OZ_MMA_MAX_SLICES) return GPB_ERR_UNSUPPORTED;
   std::lock_guard<std::mutex> lock(g_oz_mutex);
   int rc = GPB_OK;
   int dev = 0;

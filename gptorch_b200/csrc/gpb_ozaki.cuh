@@ -30,13 +30,21 @@ int gemm_ozaki_nt(int m, int n, int k, double alpha, const double* A, long lda, 
 // Engines.  GPB_OZAKI / gpb_ozaki_config: slices of the library engine (cuBLASLt int8 products, 0 = off, the default).
 // GPB_I8MMA / gpb_i8mma_config: slices of the fused tcgen05 kernel (gpb_ozaki_mma.cu; 8 by default, 0 = FP64 DMMA).
 // gemm_ozaki_nt_ex runs the library engine while ozaki_slices() > 0 and the fused kernel otherwise; the Cholesky's
-// updates use sliced_slices() = ozaki_slices() if that is > 0, else i8mma_slices(); the inverse's use ozaki_slices().
+// updates use sliced_slices() = ozaki_slices() if that is > 0, else i8mma_slices(); the inverse's use inverse_slices(n).
 int ozaki_slices();
 void ozaki_set_slices(int s);
 int i8mma_slices();
 void i8mma_set_slices(int s);
 int sliced_slices();
-constexpr int OZ_MMA_MAX_SLICES = 8, OZ_MMA_DEFAULT_SLICES = 8;
+// Slices of the blocked inverse's products (gpb_chol.cu) at order n: ozaki_slices() if that is > 0, else OZ_INV_SLICES
+// while the fused engine is on, else 0 (FP64 DMMA); always 0 when n is not a multiple of 16, so that the inverse's
+// products are either all sliced or none.  The inverse takes more slices than the factor: its consumers (tr(Ky^-1 dK),
+// the predictive variance) cancel and amplify the products' norm-wise error, which shrinks 2^7 per slice (DESIGN.md
+// section 8).
+int inverse_slices(int n);
+// OZ_MMA_MAX_SLICES: what gpb_gemm_ozaki_nt and gpb_i8mma_config take on the fused engine; the kernel itself takes up to
+// OZ_MMA_MAX_TILE_SLICES (in narrower tiles, gpb_ozaki_mma.cu), which only the inverse's products use.
+constexpr int OZ_MMA_MAX_SLICES = 8, OZ_MMA_DEFAULT_SLICES = 8, OZ_MMA_MAX_TILE_SLICES = 9, OZ_INV_SLICES = 9;
 // The fused product (gpb_ozaki_mma.cu) on slices already split by gemm_ozaki_nt_ex: a8 (m rows) and b8 (n rows), both in
 // forward slice order with row pitch slices * k bytes, row scales sa / sb.
 int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const double* sa, const double* sb);

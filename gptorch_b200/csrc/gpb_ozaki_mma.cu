@@ -1,13 +1,15 @@
 // gpb_ozaki_mma.cu -- the int8-sliced FP64-equivalent product C = beta C + alpha A B^T (DESIGN.md section 8) as ONE
-// tcgen05 kernel: all weight-class sums of a 128 x 64 output tile accumulate in tensor memory, and the epilogue
+// tcgen05 kernel: all weight-class sums of a 128 x BN output tile accumulate in tensor memory, and the epilogue
 // recombines them in fp64.  Operands are the slice buffers of oz_split_kernel / oz_split_t_kernel (gpb_ozaki.cu), both
 // in the forward layout (slice s of a row at byte offset s k), with one power-of-two scale per row.
 //
 // Class u = s + t collects the products Q^A_s (Q^B_t)^T.  The B slices of one k-chunk lie in shared memory one after the
-// other (slice-major, 64 rows each), so A_s times B slices t0 .. t0 + nt - 1 is a single MMA of N = 64 nt whose output
-// columns are exactly the accumulators of the classes s + t0 .. s + t0 + nt - 1 (class u at TMEM columns 64 u .. 64 u + 63).
-// Classes u >= S are never formed.  For S = 8 one k-step of 32 bytes is 12 MMAs (N <= 256) instead of 36 of N = 64, and
-// reads A once per MMA: 120 KB of shared memory per 9.4 M MAC, inside the 128 B/clk an SM can deliver.
+// other (slice-major, BN rows each), so A_s times B slices t0 .. t0 + nt - 1 is a single MMA of N = BN nt whose output
+// columns are exactly the accumulators of the classes s + t0 .. s + t0 + nt - 1 (class u at TMEM columns BN u ..
+// BN u + BN - 1).  Classes u >= S are never formed.  The S classes of a 64-column tile fill the 512 TMEM columns at S = 8,
+// so S <= 8 uses BN = 64 and S = 9 (the blocked inverse's products, gpb_chol.cu) BN = 32.  For S = 8 one k-step of 32
+// bytes is 12 MMAs (N <= 256) instead of 36 of N = 64, and reads A once per MMA: 120 KB of shared memory per 9.4 M MAC,
+// inside the 128 B/clk an SM can deliver.  For S = 9 it is 10 MMAs (N <= 256): 85 KB per 5.9 M MAC.
 //
 // The int32 class sums are exact ((u + 1) k 4096 < 2^31, checked by the driver), and the epilogue runs the operation
 // sequence of oz_recombine_kernel (Horner from class S-1 down, then (alpha sa_i 2^-14) sb_j t, then beta C + val), so the
@@ -24,11 +26,10 @@ namespace gpb {
 
 namespace {
 
-constexpr int I8_BM = 128, I8_BN = 64;
+constexpr int I8_BM = 128;
 constexpr int I8_CH = 64;                          // k bytes per stage and slice (SWIZZLE_64B rows)
 constexpr int I8_RING_BYTES = 192 * 1024;          // shared memory given to the stage ring
 constexpr int I8_THREADS = 192;
-constexpr int I8_GROUP = 16;                       // tile rows visited together (their A rows stay in L2)
 
 struct I8Params {
   int m, n, k;
@@ -44,14 +45,24 @@ struct I8Params {
   int tiles_m, tiles_n;
 };
 
-template <int S>
+// tile width: the S class accumulators of BN columns each must fit the 512 TMEM columns
+constexpr int i8_bn(int S) { return S <= 8 ? 64 : 32; }
+
+template <int S, int BN>
 struct I8Cfg {
+  static_assert(S * BN <= 512, "the class accumulators exceed tensor memory");
   static constexpr int A_BYTES = S * I8_BM * I8_CH;
-  static constexpr int B_BYTES = S * I8_BN * I8_CH;
+  static constexpr int B_BYTES = S * BN * I8_CH;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int STAGES = std::min(8, I8_RING_BYTES / STAGE_BYTES);
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 256;
-  static constexpr int TMEM_COLS = S * I8_BN <= 256 ? 256 : 512;
+  static_assert(STAGES >= 2 && SMEM_BYTES <= 227 * 1024, "the stage ring needs two stages in shared memory");
+  static constexpr int TMEM_COLS = S * BN <= 256 ? 256 : 512;
+  static constexpr int MAX_NT = 256 / BN;         // B slices per MMA (N <= 256)
+  // tile rows visited together, column by column: the ~148 resident tiles share GROUP A blocks of 128 rows and
+  // 148 / GROUP B blocks of BN rows, streamed through L2.  32-column tiles read A twice as often per output, so they
+  // take a squarer wave (measured on B200, gpb_potri_lower at N = 32768: 636 ms with 16, 483 ms with 4).
+  static constexpr int GROUP = BN == 64 ? 16 : 4;
 };
 
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map, int x, int y, int z, uint64_t* bar) {
@@ -89,26 +100,26 @@ __device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, uint32_t (&v)[8]) {
                : "r"(taddr));
 }
 
-template <int S>
+template <int S, int BN = i8_bn(S)>
 __global__ void __launch_bounds__(I8_THREADS, 1)
 oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const I8Params p) {
-  using Cfg = I8Cfg<S>;
+  using Cfg = I8Cfg<S, BN>;
   constexpr int STAGES = Cfg::STAGES;
 
-  // ---- tile: groups of I8_GROUP tile rows, column by column inside a group --------------------------------------
+  // ---- tile: groups of Cfg::GROUP tile rows, column by column inside a group ------------------------------------
   int tm, tn;
   {
     const int t = blockIdx.x;
-    const int per_group = I8_GROUP * p.tiles_n;
+    const int per_group = Cfg::GROUP * p.tiles_n;
     const int g = t / per_group;
-    const int first = g * I8_GROUP;
-    const int rows = min(I8_GROUP, p.tiles_m - first);
+    const int first = g * Cfg::GROUP;
+    const int rows = min(Cfg::GROUP, p.tiles_m - first);
     const int l = t - g * per_group;
     tm = first + l % rows;
     tn = l / rows;
   }
-  const int m0 = tm * I8_BM, n0 = tn * I8_BN;
-  const int m_last = min(m0 + I8_BM, p.m) - 1, n_last = min(n0 + I8_BN, p.n) - 1;
+  const int m0 = tm * I8_BM, n0 = tn * BN;
+  const int m_last = min(m0 + I8_BM, p.m) - 1, n_last = min(n0 + BN, p.n) - 1;
   if (p.lower && (n0 >> 7) > ((p.gi0 + m_last) >> 7)) return;          // every column right of every row's diagonal block
 
   // ---- k range: the triangular-by-blocks operands are zero outside it (the split wrote zeros there) -------------
@@ -165,7 +176,7 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
 #pragma unroll
         for (int q = 0; q < S; ++q) tma_load_3d(a_dst + q * (I8_BM * I8_CH), &mapA, kx, q, m0, &full_bar[s]);
 #pragma unroll
-        for (int q = 0; q < S; ++q) tma_load_3d(b_dst + q * (I8_BN * I8_CH), &mapB, kx, q, n0, &full_bar[s]);
+        for (int q = 0; q < S; ++q) tma_load_3d(b_dst + q * (BN * I8_CH), &mapB, kx, q, n0, &full_bar[s]);
       }
     }
   } else if (warp == 1) {
@@ -181,12 +192,12 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
 #pragma unroll
           for (int sa = 0; sa < S; ++sa) {
 #pragma unroll
-            for (int t0 = 0; t0 < S - sa; t0 += 4) {
-              const int nt = min(4, S - sa - t0);
+            for (int t0 = 0; t0 < S - sa; t0 += Cfg::MAX_NT) {
+              const int nt = min(Cfg::MAX_NT, S - sa - t0);
               const uint64_t ad = smem_desc(a_base + sa * (I8_BM * I8_CH) + kk * 32);
-              const uint64_t bd = smem_desc(b_base + t0 * (I8_BN * I8_CH) + kk * 32);
+              const uint64_t bd = smem_desc(b_base + t0 * (BN * I8_CH) + kk * 32);
               const uint32_t acc = (it > 0 || kk > 0 || sa > 0) ? 1u : 0u;   // sa = 0 covers every class first
-              mma_i8(tmem + static_cast<uint32_t>((sa + t0) * I8_BN), ad, bd, i8_idesc(nt * I8_BN), acc);
+              mma_i8(tmem + static_cast<uint32_t>((sa + t0) * BN), ad, bd, i8_idesc(nt * BN), acc);
             }
           }
         }
@@ -216,12 +227,12 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     const double down = 1.0 / static_cast<double>(1 << 7);
     const double si = row_ok ? p.alpha * p.sa[i] * (down * down) : 0.0;
 #pragma unroll 1
-    for (int c0 = 0; c0 < I8_BN; c0 += 8) {
+    for (int c0 = 0; c0 < BN; c0 += 8) {
       uint32_t v[S][8];
       __syncwarp();
       if (nk > 0) {
 #pragma unroll
-        for (int u = 0; u < S; ++u) tmem_ld_x8(t_row + static_cast<uint32_t>(u * I8_BN + c0), v[u]);
+        for (int u = 0; u < S; ++u) tmem_ld_x8(t_row + static_cast<uint32_t>(u * BN + c0), v[u]);
         asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
       } else {
 #pragma unroll
@@ -259,10 +270,11 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
 
 template <int S>
 int launch_s(const CUtensorMap& mapA, const CUtensorMap& mapB, const I8Params& p, cudaStream_t stream) {
+  using Cfg = I8Cfg<S, i8_bn(S)>;
   static std::atomic<int> smem_state[GPB_MAX_DEVICES];
-  if (int rc = ensure_dynamic_smem(oz_mma_kernel<S>, I8Cfg<S>::SMEM_BYTES, smem_state)) return rc;
+  if (int rc = ensure_dynamic_smem(oz_mma_kernel<S>, Cfg::SMEM_BYTES, smem_state)) return rc;
   const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
-  oz_mma_kernel<S><<<static_cast<unsigned>(tiles), I8_THREADS, I8Cfg<S>::SMEM_BYTES, stream>>>(mapA, mapB, p);
+  oz_mma_kernel<S><<<static_cast<unsigned>(tiles), I8_THREADS, Cfg::SMEM_BYTES, stream>>>(mapA, mapB, p);
   count_launch();
   GPB_CUDA_CHECK(cudaGetLastError());
   return GPB_OK;
@@ -272,10 +284,12 @@ int launch_s(const CUtensorMap& mapA, const CUtensorMap& mapB, const I8Params& p
 
 int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const double* sa, const double* sb) {
   const int S = x.slices;
+  if (S < 2 || S > OZ_MMA_MAX_TILE_SLICES) return GPB_ERR_UNSUPPORTED;
+  const int bn = i8_bn(S);
   CUtensorMap mapA, mapB;
   int rc = make_tmap_i8_slices(&mapA, a8, x.m, x.k, S, I8_CH, I8_BM);
   if (rc) return rc;
-  rc = make_tmap_i8_slices(&mapB, b8, x.n, x.k, S, I8_CH, I8_BN);
+  rc = make_tmap_i8_slices(&mapB, b8, x.n, x.k, S, I8_CH, bn);
   if (rc) return rc;
   I8Params p;
   p.m = x.m; p.n = x.n; p.k = x.k;
@@ -286,7 +300,7 @@ int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const do
   p.a_trans = x.a_trans; p.a_tri = x.a_tri; p.a_row0 = x.a_row0; p.a_col0 = x.a_col0;
   p.b_trans = x.b_trans; p.b_tri = x.b_tri; p.b_row0 = x.b_row0; p.b_col0 = x.b_col0;
   p.tiles_m = (x.m + I8_BM - 1) / I8_BM;
-  p.tiles_n = (x.n + I8_BN - 1) / I8_BN;
+  p.tiles_n = (x.n + bn - 1) / bn;
   switch (S) {
     case 2: return launch_s<2>(mapA, mapB, p, x.stream);
     case 3: return launch_s<3>(mapA, mapB, p, x.stream);
@@ -295,6 +309,7 @@ int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const do
     case 6: return launch_s<6>(mapA, mapB, p, x.stream);
     case 7: return launch_s<7>(mapA, mapB, p, x.stream);
     case 8: return launch_s<8>(mapA, mapB, p, x.stream);
+    case 9: return launch_s<9>(mapA, mapB, p, x.stream);
   }
   return GPB_ERR_UNSUPPORTED;
 }

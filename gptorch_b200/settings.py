@@ -51,8 +51,9 @@ svgp_quadratic_form = "auto"
 
 def int8_sliced_products(slices=None):
     """Slices of the FP64-equivalent int8 products that run the large O(N^3) trailing updates of the Cholesky factor
-    (DESIGN.md section 8; the inverse stays on the FP64 DMMA engine): 8 by default, 2..8 allowed, 0 = the FP64 DMMA
-    engine.  With an argument it sets the value for the process (and returns the previous one); without, it only
+    (DESIGN.md section 8): 8 by default, 2..8 allowed, 0 = the FP64 DMMA engine.  While it is above 0 the blocked
+    inverse's products run sliced too, at a fixed 9 slices (its consumers cancel, so it keeps one more); 0 returns both
+    to the FP64 DMMA engine.  With an argument it sets the value for the process (and returns the previous one); without, it only
     queries.  The environment variable GPB_I8MMA sets the initial value."""
     from . import _native
     return _native.i8mma_config(-1 if slices is None else int(slices))

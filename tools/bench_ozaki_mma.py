@@ -1,7 +1,8 @@
 """Times the three engines of the O(N^3) products side by side in one process, alternating them shape by shape: the FP64
 DMMA engine, the library int8-sliced engine (cuBLASLt products, gpb_ozaki_config) and the fused tcgen05 int8-sliced
-kernel (gpb_i8mma_config, the default).  Shapes: the SYRK-shaped trailing update C -= P P^T (lower blocks, m = 30720,
-k = 2048) and gpb_potrf_lower / gpb_potri_lower at N = 16384 and 32768.  For each: time (median of the repetitions), int8
+kernel (gpb_i8mma_config, the default; its inverse runs at INVERSE_SLICES in 32-column tiles, whatever --slices says).
+Shapes: the SYRK-shaped trailing update C -= P P^T (lower blocks, m = 30720, k = 2048) and gpb_potrf_lower /
+gpb_potri_lower at N = 16384 and 32768.  For each: time (median of the repetitions), int8
 TOP/s (the slice products the engine issues), FP64-equivalent TFLOP/s, peak device memory, plus the card's name, power
 limit and maximum SM clock.
 
@@ -19,6 +20,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."
 from gptorch_b200 import _native as nv  # noqa: E402
 
 ENGINES = ("dmma", "library", "native")
+INVERSE_SLICES = 9          # the fused engine's slice count for gpb_potri_lower's products (csrc/gpb_ozaki.cuh)
 
 
 def card():
@@ -116,6 +118,10 @@ def factor_case(n, slices, reps):
              "potri_all_ms": state["potri"], "device_used_bytes": device_used_bytes(),
              "potrf_fp64_equiv_tflops": n ** 3 / 3.0 / med["potrf"] * 1e-9,
              "potri_fp64_equiv_tflops": 2.0 * n ** 3 / 3.0 / med["potri"] * 1e-9}
+        if eng != "dmma":
+            s_inv = INVERSE_SLICES if eng == "native" else slices
+            r["potri_slices"] = s_inv
+            r["potri_int8_tops"] = r["potri_fp64_equiv_tflops"] * s_inv * (s_inv + 1) / 2
         res[eng] = r
         use("dmma", slices)
     return res
