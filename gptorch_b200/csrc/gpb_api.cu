@@ -144,7 +144,7 @@ static inline int kuf_k_per_split(int rows) {
 #pragma GCC visibility push(default)
 extern "C" {
 
-int gpb_version(void) { return 104; }
+int gpb_version(void) { return 105; }
 const char* gpb_last_error(void) { return last_error(); }
 int gpb_block_size(void) { return NB; }
 long gpb_launch_count(void) { return launch_count(); }

@@ -95,6 +95,17 @@ __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
 
+// Thread-block clusters: this CTA's rank in its cluster, and a barrier over every thread of the cluster that also orders
+// shared-memory writes (mbarrier initialisation included) before the peers' reads.
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
 // D(8x8) += A(8x4,row) * B(4x8,col), fp64.  Lane l holds A[l>>2][l&3], B[l&3][l>>2], C[l>>2][2*(l&3)+{0,1}].
 __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
   asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"

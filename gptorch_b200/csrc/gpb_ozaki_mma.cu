@@ -7,17 +7,24 @@
 // other (slice-major, BN rows each), so A_s times B slices t0 .. t0 + nt - 1 is a single MMA of N = BN nt whose output
 // columns are exactly the accumulators of the classes s + t0 .. s + t0 + nt - 1 (class u at TMEM columns BN u ..
 // BN u + BN - 1).  Classes u >= S are never formed.  The S classes of a 64-column tile fill the 512 TMEM columns at S = 8,
-// so S <= 8 uses BN = 64 and S = 9 (the blocked inverse's products, gpb_chol.cu) BN = 32.  For S = 8 one k-step of 32
+// so S <= 8 uses BN = 64 and S = 9 (the blocked inverse's products, gpb_chol.cu) BN = 48.  For S = 8 one k-step of 32
 // bytes is 12 MMAs (N <= 256) instead of 36 of N = 64, and reads A once per MMA: 120 KB of shared memory per 9.4 M MAC,
-// inside the 128 B/clk an SM can deliver.  For S = 9 it is 10 MMAs (N <= 256): 85 KB per 5.9 M MAC.
+// inside the 128 B/clk an SM can deliver.  For S = 9 it is 13 MMAs (N <= 240): 120 KB per 8.8 M MAC.
+//
+// A narrow tile reloads the same 128 A rows for every BN output columns, and A is most of the operand bytes (S = 9:
+// 36.9 KB of A and 13.8 KB of B per 32-byte k-step).  So CTAs run in clusters of two that take neighbouring tiles of one
+// tile row: each loads its own B slices and half of the A slices, the latter multicast into both CTAs' shared memory,
+// which halves the A traffic out of L2.  Both CTAs of a pair run the same k loop over the union of their two k-ranges
+// (a 48-column pair can straddle two 128-blocks; the split wrote zeros in the triangular operands' zero blocks, so the
+// extra k-steps add zero to the exact sums).
 //
 // The int32 class sums are exact ((u + 1) k 4096 < 2^31, checked by the driver), and the epilogue runs the operation
 // sequence of oz_recombine_kernel (Horner from class S-1 down, then (alpha sa_i 2^-14) sb_j t, then beta C + val), so the
 // result is bitwise the one of the unfused library engine.
 //
 // Roles (192 threads): warp 0 issues the TMA loads into a ring of stages, warp 1 allocates TMEM and one lane issues the
-// MMAs (tcgen05.commit releases each stage and finally signals the epilogue), warps 2-5 read the class planes with
-// tcgen05.ld (warp w owns TMEM lanes 32 (w % 4) ..) and write C.
+// MMAs (tcgen05.commit releases each stage in both CTAs of the pair and finally signals the epilogue), warps 2-5 read the
+// class planes with tcgen05.ld (warp w owns TMEM lanes 32 (w % 4) ..) and write C.
 #include "gpb_common.cuh"
 #include "gpb_ozaki.cuh"
 #include <algorithm>
@@ -28,7 +35,7 @@ namespace {
 
 constexpr int I8_BM = 128;
 constexpr int I8_CH = 64;                          // k bytes per stage and slice (SWIZZLE_64B rows)
-constexpr int I8_RING_BYTES = 192 * 1024;          // shared memory given to the stage ring
+constexpr int I8_RING_BYTES = 198 * 1024;          // shared memory given to the stage ring (two stages at S = 9)
 constexpr int I8_THREADS = 192;
 
 struct I8Params {
@@ -42,11 +49,11 @@ struct I8Params {
   double* Cdiag;
   int a_trans, a_tri, a_row0, a_col0;
   int b_trans, b_tri, b_row0, b_col0;
-  int tiles_m, tiles_n;
+  int tiles_m, tiles_n, pairs_n;
 };
 
-// tile width: the S class accumulators of BN columns each must fit the 512 TMEM columns
-constexpr int i8_bn(int S) { return S <= 8 ? 64 : 32; }
+// tile width: the S class accumulators of BN columns each must fit the 512 TMEM columns (S = 9: 432 of them)
+constexpr int i8_bn(int S) { return S <= 8 ? 64 : 48; }
 
 template <int S, int BN>
 struct I8Cfg {
@@ -59,9 +66,8 @@ struct I8Cfg {
   static_assert(STAGES >= 2 && SMEM_BYTES <= 227 * 1024, "the stage ring needs two stages in shared memory");
   static constexpr int TMEM_COLS = S * BN <= 256 ? 256 : 512;
   static constexpr int MAX_NT = 256 / BN;         // B slices per MMA (N <= 256)
-  // tile rows visited together, column by column: the ~148 resident tiles share GROUP A blocks of 128 rows and
-  // 148 / GROUP B blocks of BN rows, streamed through L2.  32-column tiles read A twice as often per output, so they
-  // take a squarer wave (measured on B200, gpb_potri_lower at N = 32768: 636 ms with 16, 483 ms with 4).
+  // tile rows visited together, pair column by pair column: the ~74 resident pairs share GROUP A blocks of 128 rows
+  // and 74 / GROUP B blocks of 2 BN rows, streamed through L2.
   static constexpr int GROUP = BN == 64 ? 16 : 4;
 };
 
@@ -69,6 +75,16 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst),
       "l"(map), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar))
+      : "memory");
+}
+
+// The same box written to the same shared-memory offset in both CTAs of the pair; each CTA's barrier at `bar`'s offset
+// receives the bytes.
+__device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const CUtensorMap* map, int x, int y, int z, uint64_t* bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
+      " [%0], [%1, {%2, %3, %4}], [%5], %6;" ::"r"(dst),
+      "l"(map), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar)), "h"(static_cast<uint16_t>(3))
       : "memory");
 }
 
@@ -94,6 +110,13 @@ __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// Arrives on the barrier at `bar`'s offset in both CTAs of the pair once this CTA's MMAs so far have completed.
+__device__ __forceinline__ void mma_commit_pair(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                   smem_u32(bar)), "h"(static_cast<uint16_t>(3))
+               : "memory");
+}
+
 __device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
@@ -106,21 +129,27 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
   using Cfg = I8Cfg<S, BN>;
   constexpr int STAGES = Cfg::STAGES;
 
-  // ---- tile: groups of Cfg::GROUP tile rows, column by column inside a group ------------------------------------
-  int tm, tn;
+  // ---- tile: cluster c is tile row tm and pair column pc, CTA rank r takes tile column 2 pc + r.  Pairs go in groups
+  // of Cfg::GROUP tile rows, pair column by pair column inside a group ----------------------------------------------
+  const uint32_t rank = cluster_ctarank();
+  int tm, pc;
   {
-    const int t = blockIdx.x;
-    const int per_group = Cfg::GROUP * p.tiles_n;
-    const int g = t / per_group;
+    const int c = blockIdx.x >> 1;
+    const int per_group = Cfg::GROUP * p.pairs_n;
+    const int g = c / per_group;
     const int first = g * Cfg::GROUP;
     const int rows = min(Cfg::GROUP, p.tiles_m - first);
-    const int l = t - g * per_group;
+    const int l = c - g * per_group;
     tm = first + l % rows;
-    tn = l / rows;
+    pc = l / rows;
   }
+  const int tn = 2 * pc + static_cast<int>(rank);
+  const bool phantom = tn >= p.tiles_n;                        // odd tiles_n: the last pair's second tile stores nothing
   const int m0 = tm * I8_BM, n0 = tn * BN;
-  const int m_last = min(m0 + I8_BM, p.m) - 1, n_last = min(n0 + BN, p.n) - 1;
-  if (p.lower && (n0 >> 7) > ((p.gi0 + m_last) >> 7)) return;          // every column right of every row's diagonal block
+  const int m_last = min(m0 + I8_BM, p.m) - 1;
+  // the pair's columns: the k range and the early return below are the pair's, so that both CTAs take them alike
+  const int pn0 = 2 * pc * BN, pn_last = min(pn0 + 2 * BN, p.n) - 1;
+  if (p.lower && (pn0 >> 7) > ((p.gi0 + m_last) >> 7)) return;        // every column right of every row's diagonal block
 
   // ---- k range: the triangular-by-blocks operands are zero outside it (the split wrote zeros there) -------------
   int k_lo = 0, k_hi = p.k;
@@ -129,8 +158,8 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     else k_lo = max(k_lo, ((p.a_row0 + m0) / NB) * NB - p.a_col0);
   }
   if (p.b_tri) {
-    if (p.b_trans) k_hi = min(k_hi, ((p.b_col0 + n_last) / NB + 1) * NB - p.b_row0);
-    else k_lo = max(k_lo, ((p.b_row0 + n0) / NB) * NB - p.b_col0);
+    if (p.b_trans) k_hi = min(k_hi, ((p.b_col0 + pn_last) / NB + 1) * NB - p.b_row0);
+    else k_lo = max(k_lo, ((p.b_row0 + pn0) / NB) * NB - p.b_col0);
   }
   k_lo &= ~(I8_CH - 1);
   const int nk = k_hi > k_lo ? (k_hi - k_lo + I8_CH - 1) / I8_CH : 0;
@@ -147,7 +176,7 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
+      mbar_init(&empty_bar[s], 2);                            // released by the MMAs of both CTAs
     }
     mbar_init(acc_bar, 1);
     mbar_fence_init();
@@ -158,7 +187,7 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
+  cluster_sync();                                              // the peer's barriers are initialised before any load
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem = *tmem_slot;
 
@@ -167,17 +196,23 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     if (lane == 0) {
       tma_prefetch_desc(&mapA);
       tma_prefetch_desc(&mapB);
+      // a stage is refilled once both CTAs' MMAs have released it: this CTA writes A into the peer's copy too
       for (int it = 0; it < nk; ++it) {
         const int s = it % STAGES;
         mbar_wait(&empty_bar[s], ((it / STAGES) & 1) ^ 1u);
-        mbar_expect_tx(&full_bar[s], Cfg::STAGE_BYTES);
+        mbar_expect_tx(&full_bar[s], phantom ? Cfg::A_BYTES : Cfg::STAGE_BYTES);
         const uint32_t a_dst = smem_base + s * Cfg::STAGE_BYTES, b_dst = a_dst + Cfg::A_BYTES;
         const int kx = k_lo + it * I8_CH;
 #pragma unroll
-        for (int q = 0; q < S; ++q) tma_load_3d(a_dst + q * (I8_BM * I8_CH), &mapA, kx, q, m0, &full_bar[s]);
+        for (int q = static_cast<int>(rank); q < S; q += 2)
+          tma_load_3d_pair(a_dst + q * (I8_BM * I8_CH), &mapA, kx, q, m0, &full_bar[s]);
+        if (!phantom) {
 #pragma unroll
-        for (int q = 0; q < S; ++q) tma_load_3d(b_dst + q * (BN * I8_CH), &mapB, kx, q, n0, &full_bar[s]);
+          for (int q = 0; q < S; ++q) tma_load_3d(b_dst + q * (BN * I8_CH), &mapB, kx, q, n0, &full_bar[s]);
+        }
       }
+      // wait for the last releases of every stage: after this no arrival from the peer is still in flight to this CTA
+      for (int it = nk; it < nk + STAGES; ++it) mbar_wait(&empty_bar[it % STAGES], ((it / STAGES) & 1) ^ 1u);
     }
   } else if (warp == 1) {
     // =============================== MMA issue ================================================
@@ -201,7 +236,7 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             }
           }
         }
-        mma_commit(&empty_bar[s]);
+        mma_commit_pair(&empty_bar[s]);
       }
       mma_commit(acc_bar);
     }
@@ -261,7 +296,7 @@ oz_mma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
   }
 
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
+  cluster_sync();                                              // no CTA leaves while its peer may still signal it
   if (warp == 1) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(Cfg::TMEM_COLS));
@@ -273,8 +308,19 @@ int launch_s(const CUtensorMap& mapA, const CUtensorMap& mapB, const I8Params& p
   using Cfg = I8Cfg<S, i8_bn(S)>;
   static std::atomic<int> smem_state[GPB_MAX_DEVICES];
   if (int rc = ensure_dynamic_smem(oz_mma_kernel<S>, Cfg::SMEM_BYTES, smem_state)) return rc;
-  const long tiles = static_cast<long>(p.tiles_m) * p.tiles_n;
-  oz_mma_kernel<S><<<static_cast<unsigned>(tiles), I8_THREADS, Cfg::SMEM_BYTES, stream>>>(mapA, mapB, p);
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(static_cast<unsigned>(2L * p.tiles_m * p.pairs_n));
+  cfg.blockDim = dim3(I8_THREADS);
+  cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  GPB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, oz_mma_kernel<S>, mapA, mapB, p));
   count_launch();
   GPB_CUDA_CHECK(cudaGetLastError());
   return GPB_OK;
@@ -301,6 +347,7 @@ int ozaki_mma_launch(const OzEx& x, const int8_t* a8, const int8_t* b8, const do
   p.b_trans = x.b_trans; p.b_tri = x.b_tri; p.b_row0 = x.b_row0; p.b_col0 = x.b_col0;
   p.tiles_m = (x.m + I8_BM - 1) / I8_BM;
   p.tiles_n = (x.n + bn - 1) / bn;
+  p.pairs_n = (p.tiles_n + 1) / 2;
   switch (S) {
     case 2: return launch_s<2>(mapA, mapB, p, x.stream);
     case 3: return launch_s<3>(mapA, mapB, p, x.stream);

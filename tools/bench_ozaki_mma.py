@@ -3,8 +3,9 @@ DMMA engine, the library int8-sliced engine (cuBLASLt products, gpb_ozaki_config
 kernel (gpb_i8mma_config, the default; its inverse runs at INVERSE_SLICES in 32-column tiles, whatever --slices says).
 Shapes: the SYRK-shaped trailing update C -= P P^T (lower blocks, m = 30720, k = 2048) and gpb_potrf_lower /
 gpb_potri_lower at N = 16384 and 32768.  For each: time (median of the repetitions), int8
-TOP/s (the slice products the engine issues), FP64-equivalent TFLOP/s, peak device memory, plus the card's name, power
-limit and maximum SM clock.
+TOP/s of every shape on the sliced engines (the whole shape's FP64-equivalent flops times the S(S+1)/2 class products;
+for potrf and potri this counts the DMMA panels as if sliced, so it slightly overstates the products' rate),
+FP64-equivalent TFLOP/s, peak device memory, plus the card's name, power limit and maximum SM clock.
 
     python tools/bench_ozaki_mma.py [--reps R] [--slices S] [--out FILE]
 """
@@ -121,6 +122,7 @@ def factor_case(n, slices, reps):
         if eng != "dmma":
             s_inv = INVERSE_SLICES if eng == "native" else slices
             r["potri_slices"] = s_inv
+            r["potrf_int8_tops"] = r["potrf_fp64_equiv_tflops"] * slices * (slices + 1) / 2
             r["potri_int8_tops"] = r["potri_fp64_equiv_tflops"] * s_inv * (s_inv + 1) / 2
         res[eng] = r
         use("dmma", slices)
